@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                    # this repo's CUDA path, BASELINE.json configs[1]
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's CPU path (restated), same config
     python bench.py --config 3|4|5 ...                               # the other BASELINE.json configs (see CONFIGS)
+    python bench.py ... --dump-outputs DIR                           # + what the last timed step computed, as DIR/<name>.npy
 
 Prints ONE JSON line (rank 0).  `config` is identical in both arms (it names the workload, nothing else); how each arm
 ran it is under `detail`.  See DESIGN.md "Measurement" for every field.
@@ -76,6 +77,25 @@ def ncu_traffic():
         return None
     d = json.load(open(p))
     return d.get("dram_bytes_read", 0) + d.get("dram_bytes_write", 0)
+
+
+DUMP_BYTES = 60 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy, float32 kept and everything else as float64, at most DUMP_BYTES in all:
+    when the arrays together are larger, each one over its share is replaced by a fixed, seeded sample of its elements
+    (flattened), so that two runs with the same arguments write the same elements and can be compared one to one."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in arrays.items()}
+    share = DUMP_BYTES // len(arrays)
+    over = sum(a.nbytes for a in arrays.values()) > DUMP_BYTES
+    for name, a in arrays.items():
+        if over and a.nbytes > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -307,9 +327,8 @@ def run_train(args, rank, world, local_rank, dev):
         if gather is not None:
             gather(xx, yy)
         if mode == "none":
-            eng.train_step_graph(xx, yy, args.dropout)
-        else:
-            lcn_dist.dp_train_step(eng, xx, yy, args.dropout, mode=mode, graph=not args.no_graph)
+            return eng.train_step_graph(xx, yy, args.dropout)
+        return lcn_dist.dp_train_step(eng, xx, yy, args.dropout, mode=mode, graph=not args.no_graph)
 
     for _ in range(max(args.warmup, 3)):
         step(xd, yd)
@@ -323,10 +342,13 @@ def run_train(args, rank, world, local_rank, dev):
     for a, b in evs:
         flush.zero_()
         a.record()
-        step(xd, yd)
+        loss, lr = step(xd, yd)
         b.record()
     barrier()
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
+    if args.dump_outputs and rank == 0:
+        # what the caller of the last timed step receives (loss, learning rate) and the parameters it leaves behind
+        dump_outputs(args.dump_outputs, {"loss": loss.cpu().numpy(), "lr": np.array([lr]), "params": eng.params.cpu().numpy()})
     # ---- end to end through the public API: every step copies ITS inputs from pinned host memory to the device,
     # runs the step and reads the loss back into pinned host memory.  The input copy of step i+1 runs on a copy
     # stream into the other of two device buffers while step i computes (what an input pipeline does); the host
@@ -550,7 +572,7 @@ def run_config3(args, rank, world, local_rank, dev):
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
-    reps = max(1, min(args.steps, 3))
+    reps = args.steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     t0 = time.perf_counter()
@@ -570,6 +592,8 @@ def run_config3(args, rank, world, local_rank, dev):
     dev_ms, wall = t.tolist()
     if rank != 0:
         return None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"eval_sums": s.numpy()})
     tf_burst, tf_sust, hbm, how = measured_peaks()
     c = CONFIGS[3]
     fwd_flop = fwd_flop_per_pose(nnz_of(c["mask"], c["knn"]), c["layers"], c["F"])
@@ -608,7 +632,7 @@ def run_config5(args, rank, world, local_rank, dev):
     x, y = synth_xy(B, seed=1234)
     xd, yd = torch.as_tensor(x).to(dev), torch.as_tensor(y).to(dev)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
-    sweep, head = [], None
+    sweep, head, outputs = [], None, {}
     sampler = ClockSampler(local_rank)
     sampler.start()
     for knn in (1, 2, 3, 17):
@@ -618,13 +642,17 @@ def run_config5(args, rank, world, local_rank, dev):
         for _ in range(max(args.warmup, 3)):
             eng.train_step_graph(xd, yd, args.dropout)
         torch.cuda.synchronize()
-        reps = max(5, min(args.steps, 20))
+        reps = args.steps
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(reps)]
         for a, b in ev:
             flush.zero_()
-            a.record(); eng.train_step_graph(xd, yd, args.dropout); b.record()
+            a.record(); loss, lr = eng.train_step_graph(xd, yd, args.dropout); b.record()
         torch.cuda.synchronize()
         ms = sum(a.elapsed_time(b) for a, b in ev) / reps
+        if args.dump_outputs:
+            tag = "full" if knn == 17 else knn
+            outputs.update({f"knn{tag}_loss": loss.cpu().numpy(), f"knn{tag}_lr": np.array([lr]),
+                            f"knn{tag}_params": eng.params.cpu().numpy()})
         st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
         call = lambda: L.check(eng.lib.lcn_layer_gemm(eng.h, eng.params.data_ptr(), eng.ws.data_ptr(), eng.ws.numel(), B, B, 2, 0, st))
         call()
@@ -644,6 +672,8 @@ def run_config5(args, rank, world, local_rank, dev):
         torch.cuda.empty_cache()
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     row, reps = head
     return {"metric": "poses/sec (LCN train step)", "value": row["train_poses_per_s"], "unit": "poses/s", "n_gpus": 1,
             "steps": reps, "warmup": max(args.warmup, 3), "ms_per_step": row["train_ms"], "higher_is_better": True,
@@ -686,7 +716,13 @@ def main():
     ap.add_argument("--infer-poses", type=int, default=1 << 22, help="poses per GPU of the secondary resident inference+eval leg (0: skip)")
     ap.add_argument("--total-poses", type=int, default=1 << 26, help="--config 3: poses of the whole job (sharded over the GPUs)")
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of CUDA-graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy "
+                                                          "(float32 / float64, at most 60 MiB in all; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm; --impl reference has none to write")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))

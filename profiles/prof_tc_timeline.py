@@ -1,6 +1,6 @@
-import ctypes as C, sys, numpy as np, torch
-NB = int(__import__("os").environ.get("NB", "4096"))
-sys.path.insert(0,'/root/repo')
+import ctypes as C, os, sys, numpy as np, torch
+NB = int(os.environ.get("NB", "4096"))
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from tests.gpu_helpers import make_pair, synth_xy, dev
 from lcn_pose_b200 import _lib as L
 eng,cfg,p = make_pair(L=3, knn=3, path='bf16')

@@ -1,11 +1,11 @@
 """Generate golden vectors by running the REFERENCE's own NumPy functions.
 
-Run in the build container only (needs /root/reference, which does not exist on the GPU box):
+Needs a checkout of the reference (adgx/lcn-pose), no GPU:
 
-    python tests/golden/make_golden.py
+    LCN_REFERENCE_DIR=/path/to/lcn-pose python tests/golden/make_golden.py
 
 Imports tools/params_help.py, tools/filter_hub.py, tools/tools.py, tools/data.py and
-network/models_att.get_exponential_matrix from /root/reference with tensorflow / matplotlib /
+network/models_att.get_exponential_matrix from that checkout with tensorflow / matplotlib /
 h5py / prettytable stubbed in sys.modules (they are imported at module top but not used by
 the functions called here) and writes tests/golden/reference_numpy.npz.
 """
@@ -17,7 +17,7 @@ import types
 
 import numpy as np
 
-REF = "/root/reference"
+REF = os.environ.get("LCN_REFERENCE_DIR")
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
@@ -43,6 +43,8 @@ def _stub(name):
 
 
 def import_reference():
+    if not REF:
+        sys.exit("set LCN_REFERENCE_DIR to a checkout of the reference")
     for n in ["tensorflow", "matplotlib", "matplotlib.pyplot", "mpl_toolkits", "mpl_toolkits.mplot3d",
               "h5py", "prettytable", "cv2"]:
         _stub(n)

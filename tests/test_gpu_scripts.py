@@ -2,11 +2,10 @@
 
 Two tests:
  * test_reference_scripts_run_unmodified -- executes the reference's OWN script source (train.py, inference.py,
-   evaluate.py read from /root/reference at test time, not copied) with `shims/` (+ `shims/optional_stubs/`) in front
-   of sys.path, __file__ relocated to a scratch root so that their `experiment/` and `dataset/` live there, and
-   sys.argv set to the flags a user would pass.  Needs BOTH a GPU and the reference checkout, which never coincide in
-   this project's infrastructure (the GPU box has no /root/reference, the build container no GPU): it is the proof for
-   whoever has both, and skips otherwise.
+   evaluate.py read at test time from the checkout LCN_REFERENCE_DIR names, not copied) with `shims/`
+   (+ `shims/optional_stubs/`) in front of sys.path, __file__ relocated to a scratch root so that their `experiment/`
+   and `dataset/` live there, and sys.argv set to the flags a user would pass.  Needs BOTH a GPU and a checkout of the
+   reference: it is the proof for whoever has both, and skips otherwise.
  * test_script_call_sequences_through_the_shims -- the same module-level calls the three scripts make, in their order
    (cited line by line), on synthetic pickles in the tools/gendb.py:66-81 schema.  Runs on the GPU box.  Checks the
    artefacts the scripts exchange (checkpoints, result.pkl) and the final MPJPE tables against the float64 oracle."""
@@ -26,7 +25,7 @@ from oracle import lcn_oracle as O
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = os.environ.get("LCN_REFERENCE_DIR")
 FX, FY, CX, CY = 1145.05, 1143.78, 512.54, 515.45
 
 
@@ -80,7 +79,7 @@ def _write_datasets(root):
     return sets
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference checkout exists in the build container only")
+@pytest.mark.skipif(not REF, reason="needs a checkout of the reference named by LCN_REFERENCE_DIR")
 def test_reference_scripts_run_unmodified(tmp_path):
     root = str(tmp_path)
     _write_datasets(root)
