@@ -187,7 +187,8 @@ int lcn_model_unpack_grads(lcn_model* m, const float* d_compact, float* d_grads_
  * lcn_model_backward then leaves the MEAN of the ranks' gradients in the bucket, exchanged in place by the library's own
  * kernel (in stream order; capturable into the caller's CUDA graph like every other call), so
  * lcn_model_adam_step needs no change and a data-parallel step is one graph.  Every rank must issue the same sequence of
- * lcn_model_backward calls.  BatchNorm statistics stay per GPU (== the reference at batch B per GPU).
+ * lcn_model_backward calls.  By default BatchNorm statistics stay per GPU (== the reference at batch B per GPU); see
+ * lcn_dp_sync_batch_norm for statistics of the global batch.
  * The exchange is STREAMED: the joint-pair blocks of every mid-layer weight gradient travel on a third stream of the
  * model as soon as that layer's weight-gradient GEMM has finished, under the rest of the backward pass; only the first /
  * last layer and the small tensors (< 2 % of the bucket) are exchanged after it.
@@ -198,6 +199,18 @@ float* lcn_dp_bucket(const lcn_model* m);   /* the rank's peer-mapped gradient b
 int lcn_dp_connect(lcn_model* m, const void* h_handles /* world x 64 bytes, rank order */, int rank, int world);
 int lcn_dp_world(const lcn_model* m);
 int lcn_dp_enable(lcn_model* m, int mode);
+/* Synchronised BatchNorm (off by default; on != 0 needs a connected model, off is always accepted).  With it on, every
+ * training forward pass (lcn_model_forward(training=1), one BN group = this rank's n_rows) normalises each BatchNorm
+ * layer with the mean and biased variance of ALL ranks' rows x 17 joints -- the statistics a single GPU computes on the
+ * concatenated batch -- and lcn_model_backward uses the matching global sums: dZ = gamma rstd (d - S1/N - xhat S2/N),
+ * S1 = sum over ranks and rows of d, S2 = of d xhat, N = 17 x global rows.  Each rank's gradient is then `world` times
+ * its share of the gradient of (1/world) sum_r L_r, so the bucket's mean (any lcn_dp_enable mode, or the host's own
+ * all-reduce in mode 0) is that gradient; gamma / beta gradients stay per-rank sums.  Shards may differ in size.  Every
+ * rank combines the ranks' moments in rank order in fp64, so the statistics are bit-identical across ranks.  Costs one
+ * NVLink flag round trip per BN layer in the forward and in the backward pass.  Inference keeps per-group statistics;
+ * lcn_model_forward_layers returns LCN_ESTATE while sync is on.  lcn_model_read_tensor kinds 4 / 5 return the global
+ * statistics. */
+int lcn_dp_sync_batch_norm(lcn_model* m, int on);
 
 /* (a10) ... or applies TF1 Adam directly from the raw gradients in one fused pass (models_att.py:404-409):
  * lr_t = lr*sqrt(1-b2^t)/(1-b1^t) is computed by the caller (host scalar); theta -= lr_t*m/(sqrt(v)+eps).

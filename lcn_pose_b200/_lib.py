@@ -59,6 +59,7 @@ PROTOTYPES = {
     "lcn_dp_connect": (C.c_int, [_vp, _vp, C.c_int, C.c_int]),
     "lcn_dp_world": (C.c_int, [_vp]),
     "lcn_dp_enable": (C.c_int, [_vp, C.c_int]),
+    "lcn_dp_sync_batch_norm": (C.c_int, [_vp, C.c_int]),
     "lcn_model_adam_step": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _sz, _vp, _f, _f, _f, _f, _f, _vp, _vp]),
     "lcn_layer_gemm": (C.c_int, [_vp, _vp, _vp, _sz, _i64, _i32, C.c_int, C.c_int, _vp]),
     "lcn_model_read_tensor": (C.c_int, [_vp, _vp, _sz, C.c_int, C.c_int, _i64, _i32, _vp, _vp]),

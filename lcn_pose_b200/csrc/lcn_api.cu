@@ -445,6 +445,10 @@ extern "C" int lcn_model_forward_layers(lcn_model* m, const float* d_params, voi
   LCN_REQUIRE(d_x != nullptr || (layer_begin > 0 && layer_end < m->n_lin), "the first and the last layer read d_x");
   LCN_REQUIRE(d_out != nullptr || layer_end < m->n_lin, "the last layer writes d_out");
   LCN_REQUIRE(dropout_rate >= 0.f && dropout_rate < 1.f, "dropout rate %f outside [0,1)", dropout_rate);
+  if (lcn_bn_sync_on(m)) {   // its per-layer batch statistics would disagree with the global ones of the backward pass
+    lcn_set_error("lcn_model_forward_layers: not available while synchronised BatchNorm is on (lcn_dp_sync_batch_norm)");
+    return LCN_ESTATE;
+  }
   FwdArgs a;
   a.m = m;
   a.params = d_params;

@@ -41,6 +41,27 @@
 // the epoch from device memory, so the exchange is captured into the train-step CUDA graph like any other kernel of the
 // step.  No kernel needs a peer's kernel to be co-scheduled in order to FINISH its own loads and stores; the waits are on
 // flags that the peers' stream-ordered work sets unconditionally, so a late peer delays, never deadlocks.
+//
+// Synchronised BatchNorm (lcn_dp_sync_batch_norm, off by default): every BatchNorm layer of a training step normalises
+// with the moments of the GLOBAL batch.  A step has 2 * n_bn sync points (point l: forward of BN layer l, point n_bn + l:
+// its backward), each one launch of k_bn_sync on the caller's stream:
+//
+//   forward   (n, mean, M2) per channel of this rank's rows x 17 joints (from the GEMM's fp64 sums or from k_bn_finalize)
+//             -> merged in rank order (k_bn_finalize's formula, fp64) -> (mean, rstd) of the global batch into the stat
+//             buffer that k_bn_act(_pre), the backward pass and read_tensor kinds 4 / 5 read
+//   backward  (n, sum dy, sum dy*xhat) per channel from k_bn_bwd_reduce -> summed in rank order (fp64) -> (S1 / N, S2 / N)
+//             with N = 17 x global rows, which k_bn_bwd_apply uses instead of its local sums / local count
+//
+// The BN area behind the staging slots holds, per point, one slot of 3 F doubles per rank and three flag words per rank.
+// k_bn_sync: (1) waits until consumed[pt][p] >= e - 1 for every p, (2) stores its payload into slot [pt][me] of every
+// rank with peer stores, (3) publishes ready[pt][me] = e at every rank (st.release.sys), (4) waits for ready[pt][p] >= e
+// for every p (ld.acquire.sys), merges the `world` slots in rank order -- every rank computes bit-identical statistics --
+// and (5) publishes consumed[pt][me] = e at every rank.  e = ++epoch[pt], a local counter in device memory, so the kernel
+// is captured into the train-step graph like the gradient exchange.
+// Slot-reuse invariant: a rank overwrites slot [pt][me] at rank p (epoch e) only after p has published consumed[pt] = e - 1,
+// i.e. after p's last read of that slot for epoch e - 1.  This holds with no gradient exchange between two steps (mode 0,
+// eager forward-only calls), because it rests on the point's own flags and not on the order of other kernels.  Every
+// rank must run the same sequence of training forward / backward calls while sync is on.
 #include <stdlib.h>
 
 #include <algorithm>
@@ -62,13 +83,24 @@ struct LcnDpFlags {                       // lives at the start of every rank's 
   unsigned int ticket;                    // local: CTAs of k_dp_reduce that have finished
 };
 
+// BN area (synchronised BatchNorm), behind the staging slots: LcnBnFlags[points], then double[points][world][3 F]
+struct LcnBnFlags {
+  unsigned long long ready[LCN_DP_MAX_WORLD];      // ready[p]: written by rank p -- its payload of epoch ready[p] is in slot p here
+  unsigned long long consumed[LCN_DP_MAX_WORLD];   // consumed[p]: written by rank p -- it has merged epoch consumed[p]
+  unsigned long long epoch;                        // local: uses of the point by this rank
+  unsigned long long pad[7];
+};
+
 struct LcnDp {
   int rank = 0, world = 1;
   int mode = LCN_DP_STREAMED;             // lcn_dp_enable: 0 off, 1 streamed behind the weight-gradient GEMMs, 2 one exchange at the end
   bool connected = false;
+  bool sync_bn = false;                   // lcn_dp_sync_batch_norm
   int64_t count = 0;                      // floats in the bucket (= lcn_model_param_count)
   int64_t packed = 0;                     // floats in one staging slot (= lcn_model_grad_compact_count, 16-byte rounded)
   size_t stage_off = 0, slot_bytes = 0;   // staging: `world` slots behind the bucket
+  size_t bn_off = 0, bn_slot_off = 0;     // BN area: flags of the 2 n_bn sync points, then their slots
+  int bn_points = 0, F = 0;
   size_t bytes = 0;
   char* base = nullptr;                   // own allocation
   char* peer[LCN_DP_MAX_WORLD] = {};      // mapped allocations (peer[rank] == base)
@@ -105,6 +137,108 @@ __global__ void k_dp_wait(DpFlagPtrs d) {
   }
 }
 
+__device__ __forceinline__ void bn_wait_flag(const unsigned long long* p, unsigned long long e, const char* what) {
+  unsigned long long spins = 0;
+  while (ld_acquire_sys(p) < e) {
+    if (++spins > (1ull << 28)) {          // seconds: a peer died or the ranks disagree on the call sequence
+      printf("lcn_dp: synchronised BatchNorm: wait for a peer's %s flag timed out\n", what);
+      __trap();
+    }
+  }
+}
+
+struct BnSyncArgs {                       // by-value kernel argument: one sync point
+  double* slot_at[LCN_DP_MAX_WORLD];      // slot [point][me] at rank p
+  unsigned long long* ready_at[LCN_DP_MAX_WORLD];
+  unsigned long long* consumed_at[LCN_DP_MAX_WORLD];
+  const double* slots;                    // local slots [point][0 .. world)
+  LcnBnFlags* mine;                       // local flags of the point
+  int rank, world;
+};
+
+// One CTA, thread f = channel f (F <= 256).  kind: LCN_BN_SYNC_GACC (src: double[LCN_GACC_REP][F][2] sums of x, x^2),
+// LCN_BN_SYNC_MOMENTS (src: double[F][3] (n, mean, M2) of k_bn_finalize) -> out float[F][2] (mean, rstd);
+// LCN_BN_SYNC_SUMS (src: float[F][2] (sum dy, sum dy*xhat)) -> out float[F][2] (S1 / N, S2 / N).
+__global__ void __launch_bounds__(256) k_bn_sync(BnSyncArgs s, int kind, const void* __restrict__ src,
+                                                 float* __restrict__ out, int F, double n_local) {
+  lcn_pdl_wait();    // no early trigger: the next kernel's CTAs must not sit on SMs while this one waits for the peers
+  __shared__ unsigned long long s_e;
+  const int f = threadIdx.x;
+  double a = 0.0, b = 0.0;                // forward: (mean, M2); backward: (S1, S2) of this rank's rows
+  if (f < F) {
+    if (kind == LCN_BN_SYNC_GACC) {
+      const double* g = static_cast<const double*>(src);
+      double S1 = 0.0, S2 = 0.0;
+      for (int rep = 0; rep < LCN_GACC_REP; ++rep) {
+        S1 += g[((size_t)rep * F + f) * 2];
+        S2 += g[((size_t)rep * F + f) * 2 + 1];
+      }
+      a = S1 / n_local;
+      b = fmax(S2 - S1 * a, 0.0);
+    } else if (kind == LCN_BN_SYNC_MOMENTS) {
+      const double* mo = static_cast<const double*>(src);
+      a = mo[f * 3 + 1];
+      b = mo[f * 3 + 2];
+    } else {
+      const float* su = static_cast<const float*>(src);
+      a = (double)su[f * 2];
+      b = (double)su[f * 2 + 1];
+    }
+  }
+  if (threadIdx.x == 0) s_e = s.mine->epoch + 1;
+  __syncthreads();
+  const unsigned long long e = s_e;
+  // (1) every rank has merged the previous epoch: its slot [point][me] may be overwritten
+  if ((int)threadIdx.x < s.world) bn_wait_flag(&s.mine->consumed[threadIdx.x], e - 1, "consumed");
+  __syncthreads();
+  // (2) payload into slot [point][me] of every rank, (3) ready = e at every rank
+  if (f < F) {
+    for (int p = 0; p < s.world; ++p) {
+      double* d = s.slot_at[p] + (size_t)f * 3;
+      d[0] = n_local;
+      d[1] = a;
+      d[2] = b;
+    }
+  }
+  __syncthreads();
+  if ((int)threadIdx.x < s.world) {
+    __threadfence_system();
+    st_release_sys(s.ready_at[threadIdx.x], e);
+  }
+  // (4) every rank's payload of epoch e has landed here; merge in rank order
+  if ((int)threadIdx.x < s.world) bn_wait_flag(&s.mine->ready[threadIdx.x], e, "ready");
+  __syncthreads();
+  if (f < F) {
+    const size_t stride = (size_t)F * 3;
+    double n = __ldcg(s.slots + (size_t)f * 3), x = __ldcg(s.slots + (size_t)f * 3 + 1), y = __ldcg(s.slots + (size_t)f * 3 + 2);
+    for (int p = 1; p < s.world; ++p) {
+      const double* q = s.slots + p * stride + (size_t)f * 3;
+      const double nq = __ldcg(q), xq = __ldcg(q + 1), yq = __ldcg(q + 2);
+      if (kind == LCN_BN_SYNC_SUMS) {
+        x += xq;
+        y += yq;
+        n += nq;
+      } else {                             // pairwise merge of (n, mean, M2)
+        const double nt = n + nq, d = xq - x;
+        x += d * (nq / nt);
+        y += yq + d * d * (n * nq / nt);
+        n = nt;
+      }
+    }
+    if (kind == LCN_BN_SYNC_SUMS) {
+      out[f * 2] = (float)(x / n);
+      out[f * 2 + 1] = (float)(y / n);
+    } else {
+      out[f * 2] = (float)x;
+      out[f * 2 + 1] = (float)(1.0 / sqrt(y / n + (double)LCN_BN_EPS));
+    }
+  }
+  // (5) this rank has read every slot of the point for epoch e
+  __syncthreads();
+  if ((int)threadIdx.x < s.world) st_release_sys(s.consumed_at[threadIdx.x], e);
+  if (threadIdx.x == 0) s.mine->epoch = e;
+}
+
 }  // namespace
 
 // ---- host side ----------------------------------------------------------------------------------------------------
@@ -120,7 +254,11 @@ extern "C" int lcn_dp_export(lcn_model* m, int world, void* h_handle64) {
   dp->packed = (lcn_grad_compact_count(m) + 3) & ~(int64_t)3;
   dp->stage_off = LCN_DP_FLAG_BYTES + (((size_t)dp->count * 4 + 255) & ~(size_t)255);
   dp->slot_bytes = ((size_t)dp->packed * 4 + 255) & ~(size_t)255;
-  dp->bytes = dp->stage_off + (size_t)world * dp->slot_bytes;
+  dp->bn_points = 2 * m->n_bn;
+  dp->F = m->d.F;
+  dp->bn_off = dp->stage_off + (size_t)world * dp->slot_bytes;
+  dp->bn_slot_off = dp->bn_off + ((sizeof(LcnBnFlags) * dp->bn_points + 255) & ~(size_t)255);
+  dp->bytes = dp->bn_slot_off + sizeof(double) * dp->bn_points * world * 3 * dp->F;
   // the one device allocation the library makes: peers have to map it, so it cannot come from the caller's allocator
   cudaError_t e = cudaMalloc(&dp->base, dp->bytes);
   if (e == cudaSuccess) e = cudaMemset(dp->base, 0, dp->bytes);
@@ -176,6 +314,40 @@ extern "C" int lcn_dp_enable(lcn_model* m, int on) {
   LCN_REQUIRE((m->dp != nullptr && m->dp->connected) || !on, "lcn_dp_enable: the model is not connected (lcn_dp_export / lcn_dp_connect)");
   LCN_REQUIRE(on >= 0 && on <= 2, "lcn_dp_enable: mode %d not in {0, 1, 2}", on);
   if (m->dp) m->dp->mode = on;
+  return LCN_OK;
+}
+
+extern "C" int lcn_dp_sync_batch_norm(lcn_model* m, int on) {
+  LCN_REQUIRE(m != nullptr, "null model");
+  LCN_REQUIRE((m->dp != nullptr && m->dp->connected) || !on,
+              "lcn_dp_sync_batch_norm: the model is not connected (lcn_dp_export / lcn_dp_connect)");
+  if (m->dp) m->dp->sync_bn = on != 0;
+  return LCN_OK;
+}
+
+bool lcn_bn_sync_on(const lcn_model* m) {
+  return m->dp != nullptr && m->dp->connected && m->dp->world > 1 && m->dp->sync_bn;
+}
+
+// One sync point (see the header of this file): `rows` = this rank's training batch.
+int lcn_bn_sync(const lcn_model* m, int point, int kind, const void* src, float* out, int64_t rows, cudaStream_t st) {
+  const LcnDp* dp = m->dp;
+  LCN_REQUIRE(point >= 0 && point < dp->bn_points && m->d.F == dp->F, "internal: BatchNorm sync point %d", point);
+  BnSyncArgs s;
+  memset(&s, 0, sizeof(s));
+  const size_t pt_slots = (size_t)dp->world * 3 * dp->F;     // doubles per point
+  for (int p = 0; p < dp->world; ++p) {
+    LcnBnFlags* fl = reinterpret_cast<LcnBnFlags*>(dp->peer[p] + dp->bn_off) + point;
+    s.slot_at[p] = reinterpret_cast<double*>(dp->peer[p] + dp->bn_slot_off) + point * pt_slots + (size_t)dp->rank * 3 * dp->F;
+    s.ready_at[p] = &fl->ready[dp->rank];
+    s.consumed_at[p] = &fl->consumed[dp->rank];
+  }
+  s.slots = reinterpret_cast<const double*>(dp->base + dp->bn_slot_off) + point * pt_slots;
+  s.mine = reinterpret_cast<LcnBnFlags*>(dp->base + dp->bn_off) + point;
+  s.rank = dp->rank;
+  s.world = dp->world;
+  lcn_launch(k_bn_sync, dim3(1), dim3(256), 0, st, s, kind, src, out, dp->F, (double)rows * LCN_J);
+  LCN_CHECK_LAUNCH();
   return LCN_OK;
 }
 

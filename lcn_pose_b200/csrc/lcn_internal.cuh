@@ -250,6 +250,12 @@ int lcn_dp_mode(const lcn_model* m);      // 0: no exchange; 1: streamed behind 
 int lcn_dp_exchange_units(const lcn_model* m, float* graw, int u0, int u1, int s0, int s1, int max_ctas, cudaStream_t st);
 int lcn_dp_wait(const lcn_model* m, cudaStream_t st);
 void lcn_dp_destroy(lcn_model* m);
+// synchronised BatchNorm (lcn_dp_sync_batch_norm): the source of a sync point's local moments
+#define LCN_BN_SYNC_GACC 0      // forward, double[LCN_GACC_REP][F][2] (sum x, sum x^2) of the tensor-core GEMM
+#define LCN_BN_SYNC_MOMENTS 1   // forward, double[F][3] (n, mean, M2) of k_bn_finalize
+#define LCN_BN_SYNC_SUMS 2      // backward, float[F][2] (sum dy, sum dy*xhat) of k_bn_bwd_reduce
+bool lcn_bn_sync_on(const lcn_model* m);
+int lcn_bn_sync(const lcn_model* m, int point, int kind, const void* src, float* out, int64_t rows, cudaStream_t st);
 
 // ---- launch wrappers implemented in the kernel translation units ----
 struct FwdArgs {                 // one call of the forward pass

@@ -555,9 +555,11 @@ __global__ void __launch_bounds__(256) k_first_layer(const float* __restrict__ x
 // joints (Keras BN axis=-1 on [B,17,F]: per channel over batch x joints, biased variance).
 // grid (n_groups, F/2), 256 threads = 2 channels x 128 slices.  Two-pass merge in fp64:
 //   mean = sum n_b mean_b / N ;  M2 = sum [ M2_b + n_b (mean_b - mean)^2 ]   (exact, no per-item division)
+// mom != nullptr (synchronised BatchNorm, one group): the fp64 moments (N, mean, M2) go to mom[F][3] for k_bn_sync
+// instead of (mean, rstd) to stat.
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_bn_finalize(const float* __restrict__ part, float* __restrict__ stat, int P,
-                                                     int F, int tiles_per_group, int bn_group) {
+                                                     int F, int tiles_per_group, int bn_group, double* __restrict__ mom) {
   lcn_pdl_prologue();
   __shared__ double sa[256];
   __shared__ double smean[2];
@@ -595,7 +597,11 @@ __global__ void __launch_bounds__(256) k_bn_finalize(const float* __restrict__ p
     __syncthreads();
     if (slice < off) sa[tid] += sa[tid + off * 2];
   }
-  if (slice == 0) {
+  if (slice == 0 && mom != nullptr) {
+    mom[f * 3] = ntot;
+    mom[f * 3 + 1] = mean;
+    mom[f * 3 + 2] = sa[tid];
+  } else if (slice == 0) {
     double var = sa[tid] / ntot;
     stat[((size_t)g * F + f) * 2 + 0] = (float)mean;
     stat[((size_t)g * F + f) * 2 + 1] = (float)(1.0 / sqrt(var + (double)LCN_BN_EPS));
@@ -1079,7 +1085,7 @@ __global__ void __launch_bounds__(EW_MAXT, 2) k_bn_bwd_reduce(const T* __restric
   }
 }
 
-template <typename T>
+template <typename T, bool kSync>
 __global__ void __launch_bounds__(EW_MAXT, 2) k_bn_bwd_apply(const T* __restrict__ dOut, const T* __restrict__ Z,
                                                              const uint8_t* __restrict__ keepbits,
                                                              const float* __restrict__ stat,
@@ -1088,7 +1094,7 @@ __global__ void __launch_bounds__(EW_MAXT, 2) k_bn_bwd_apply(const T* __restrict
                                                              const float* __restrict__ sums, T* __restrict__ dZ,
                                                              float* __restrict__ dbpart, float* __restrict__ dgamma,
                                                              float* __restrict__ dbeta, int P, int F, int rows_pad,
-                                                             int bn_group, float rate) {
+                                                             int bn_group, float rate, const float* __restrict__ gmean) {
   lcn_pdl_prologue();
   extern __shared__ __align__(16) float red[];   // [Y-1][P] column sums of the other row-threads
   __shared__ __align__(16) float s_a[256], s_b[256], s_c[256], s_d[256];
@@ -1096,11 +1102,19 @@ __global__ void __launch_bounds__(EW_MAXT, 2) k_bn_bwd_apply(const T* __restrict
   BnConsts k;
   bn_load_consts(stat, gamma, beta, F, f0, s_a, s_b, s_c, s_d, k);
   float m1[8], m2[8];
-  float inv_n = 1.f / ((float)bn_group * (float)LCN_J);
+  if constexpr (kSync) {         // synchronised BatchNorm: (S1, S2) / N over all ranks' rows, from k_bn_sync
 #pragma unroll
-  for (int q = 0; q < 8; ++q) {
-    m1[q] = sums[(f0 + q) * 2] * inv_n;
-    m2[q] = sums[(f0 + q) * 2 + 1] * inv_n;
+    for (int q = 0; q < 8; ++q) {
+      m1[q] = gmean[(f0 + q) * 2];
+      m2[q] = gmean[(f0 + q) * 2 + 1];
+    }
+  } else {
+    float inv_n = 1.f / ((float)bn_group * (float)LCN_J);
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+      m1[q] = sums[(f0 + q) * 2] * inv_n;
+      m2[q] = sums[(f0 + q) * 2 + 1] * inv_n;
+    }
   }
   if (blockIdx.x == 0 && threadIdx.y == 0 && (int)threadIdx.x < F / 8) {
 #pragma unroll
@@ -1782,6 +1796,11 @@ static int forward_impl(const FwdArgs& a) {
     pre_ok = lay.n_groups == 1 && per0 <= BA_R * ewy0;
   }
   const bool try_fuse = kBf && lay.training && lay.n_groups == 1 && pre_ok;
+  const bool bn_sync = lay.training && lcn_bn_sync_on(m);      // lcn_model_forward admits it only at one group
+  if (bn_sync && lay.n_groups != 1) {
+    lcn_set_error("synchronised BatchNorm: a training forward pass must be one BatchNorm group (bn_group = n_rows)");
+    return LCN_EINVAL;
+  }
   if (try_fuse) LCN_CHECK_CUDA(cudaMemsetAsync(ws + lay.off_gacc, 0, lay.gacc_stride * (size_t)n_bn, st));
   const int lb = a.layer_begin, le = a.layer_end < 0 ? m->n_lin : a.layer_end;   // linear layers [lb, le)
   for (int l = lb; l < n_bn && l < le; ++l) {
@@ -1817,8 +1836,18 @@ static int forward_impl(const FwdArgs& a) {
     LCN_CHECK_LAUNCH();
     float* stat = bn_stat(ws, lay, m, l);
     const double* gacc = fused_bn ? reinterpret_cast<const double*>(ws + lay.off_gacc + (size_t)l * lay.gacc_stride) : nullptr;
+    // synchronised BatchNorm: k_bn_finalize leaves fp64 moments in the (otherwise unused) accumulator area of the layer,
+    // k_bn_sync merges them -- or the GEMM's sums -- with the other ranks' and writes the global (mean, rstd) to stat
+    double* mom = bn_sync ? reinterpret_cast<double*>(ws + lay.off_gacc + (size_t)l * lay.gacc_stride) : nullptr;
     if (fused_bn == 0)
-    lcn_launch(k_bn_finalize, dim3(dim3(lay.n_groups, F / 2)), dim3(256), 0, st, part, stat, P, F, lay.tiles_per_group, lay.bn_group);
+    lcn_launch(k_bn_finalize, dim3(dim3(lay.n_groups, F / 2)), dim3(256), 0, st, part, stat, P, F, lay.tiles_per_group, lay.bn_group, mom);
+    if (bn_sync) {
+      LCN_CHECK_LAUNCH();
+      int rc = lcn_bn_sync(m, l, fused_bn ? LCN_BN_SYNC_GACC : LCN_BN_SYNC_MOMENTS, fused_bn ? (const void*)gacc : mom, stat,
+                           lay.n_rows, st);
+      if (rc) return rc;
+      gacc = nullptr;                  // k_bn_act_pre reads the global statistics from stat
+    }
     const T* res = L.res_from >= 0 ? reinterpret_cast<const T*>(a_buf(ws, lay, L.res_from)) : nullptr;
     const int ewy = (P / 8) * 2 <= EW_MAXT ? 2 : 1;
     uint8_t* keepbits = (lay.training && a.dropout_rate > 0.f)
@@ -1891,6 +1920,7 @@ static int backward_impl(const lcn_model* m, const float* params, char* ws, cons
   // first and last layer and the small tensors (< 2 % of the bucket)
   const int dp_mode = lcn_dp_mode(m);
   const bool dp_stream = dp_mode == 1 && ax != nullptr;
+  const bool bn_sync = lcn_bn_sync_on(m);
   bool dp_forked = false;
   bool wg_pending[2] = {false, false};
   const int64_t blast = m->L[m->n_lin - 1].b_off;     // last-layer bias gradient: accumulated by k_loss_dout (caller's stream)
@@ -1970,9 +2000,17 @@ static int backward_impl(const lcn_model* m, const float* params, char* ws, cons
     {
       lcn_launch(k_bn_bwd_reduce<T>, dim3(eg), dim3(dim3(P / 8, ewy)), red_smem, st, D(cur), Z, keepbits, stat, params + L.gamma_off,
                                                                params + L.beta_off, sums, P, F, lay.bn_group, rate);
-      lcn_launch(k_bn_bwd_apply<T>, dim3(eg), dim3(dim3(P / 8, ewy)), (size_t)ewy * P * sizeof(float), st, 
+      float* gmean = nullptr;          // synchronised BatchNorm: (S1, S2) / N of all ranks, in the layer's accumulator area
+      if (bn_sync) {
+        LCN_CHECK_LAUNCH();
+        gmean = reinterpret_cast<float*>(ws + lay.off_gacc + (size_t)l * lay.gacc_stride);
+        int rc = lcn_bn_sync(m, m->n_bn + l, LCN_BN_SYNC_SUMS, sums, gmean, lay.n_rows, st);
+        if (rc) return rc;
+      }
+      lcn_launch(bn_sync ? k_bn_bwd_apply<T, true> : k_bn_bwd_apply<T, false>, dim3(eg), dim3(dim3(P / 8, ewy)), (size_t)ewy * P * sizeof(float), st,
           D(cur), Z, keepbits, stat, params + L.gamma_off, params + L.beta_off, sums, dZ,
-          reinterpret_cast<float*>(ws + lay.off_dbpart) + (size_t)l * eg * P, graw + L.gamma_off, graw + L.beta_off, P, F, (int)lay.rows_pad, lay.bn_group, rate);
+          reinterpret_cast<float*>(ws + lay.off_dbpart) + (size_t)l * eg * P, graw + L.gamma_off, graw + L.beta_off, P, F, (int)lay.rows_pad, lay.bn_group, rate,
+          gmean);
     }
     LCN_CHECK_LAUNCH();
     if (ax) {                        // dZ_l is ready: the side stream may start the weight gradient of layer l

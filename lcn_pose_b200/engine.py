@@ -297,6 +297,14 @@ class LcnEngine:
         L.check(self.lib.lcn_dp_enable(self.h, int(mode)))
         self._graphs.clear()
 
+    def dp_sync_batch_norm(self, on):
+        """lcn_dp_sync_batch_norm: True -> every BatchNorm layer of a training step uses the statistics of the global
+        batch (all ranks' rows), as one GPU would on the concatenated batch; False (default) -> per-rank statistics.
+        Needs a connected engine to turn on."""
+        L.check(self.lib.lcn_dp_sync_batch_norm(self.h, int(bool(on))))
+        self._graphs.clear()
+        self.sync_bn = bool(on)
+
     # ---- data-parallel exchange: only what backward produces travels (lcn_model_pack_grads) ----
     def pack_grads(self):
         """Gather the nonzero weight blocks + every other tensor of the raw-gradient bucket into self.grads_compact."""
