@@ -16,12 +16,13 @@
  *    library never synchronises the device and never allocates device memory.
  *  - every function returns 0 (LCN_OK) or a negative LCN_E* code; the message is available from
  *    lcn_last_error() (thread local).  No C++ exception crosses the boundary.
- *  - a model handle's tables (block lists, offsets) are immutable after creation.  It also owns one side stream with a
- *    few events (the weight-gradient GEMMs of lcn_model_backward and the edge-layer packs of
- *    lcn_model_prepare_weights run there, forked from and joined to the caller's stream) and, after lcn_dp_init, a
- *    communication stream: calls that use them serialise on a mutex inside the handle while they ENQUEUE (never while
- *    the GPU runs), so any number of host threads may call into the same handle with distinct streams and
- *    workspaces; one-time kernel-attribute setup is guarded by std::call_once.
+ *  - a model handle's tables (block lists, offsets) are immutable after creation.  It also owns two side streams and
+ *    a few events, created on first use: the weight-gradient GEMMs of lcn_model_backward and the edge-layer packs of
+ *    lcn_model_prepare_weights run on one, forked from and joined to the caller's stream; the data-parallel exchange
+ *    of finished weight gradients (lcn_dp_enable mode 1) runs on the other.  A call that cannot create them returns
+ *    LCN_ECUDA.  Calls that use them serialise on a mutex inside the handle while they ENQUEUE (never while the GPU
+ *    runs), so any number of host threads may call into the same handle with distinct streams and workspaces;
+ *    one-time kernel-attribute setup is guarded by std::call_once.
  *  - matrices are row-major; feature index inside a row is joint-major: column j*F + f
  *    (network/models_att.py:582); mask index is [input joint, output joint] (:583).
  */

@@ -227,19 +227,7 @@ extern "C" int lcn_model_create(const lcn_model_desc* desc, lcn_model** out) {
 extern "C" void lcn_model_destroy(lcn_model* m) {
   if (m == nullptr) return;
   lcn_dp_destroy(m);
-  if (m->aux.ready) {
-    cudaStreamDestroy(m->aux.st);
-    cudaStreamDestroy(m->aux.xst);
-    cudaEventDestroy(m->aux.ev_xdone);
-    cudaEventDestroy(m->aux.ev_go);
-    cudaEventDestroy(m->aux.ev_done);
-    cudaEventDestroy(m->aux.ev_ms);
-    cudaEventDestroy(m->aux.ev_loss);
-    for (int i = 0; i < 2; ++i) {
-      cudaEventDestroy(m->aux.ev_dz[i]);
-      cudaEventDestroy(m->aux.ev_wg[i]);
-    }
-  }
+  lcn_aux_release(m->aux);
   delete m;
 }
 extern "C" int64_t lcn_model_param_count(const lcn_model* m) { return m ? m->n_params : 0; }
@@ -333,14 +321,24 @@ extern "C" size_t lcn_model_workspace_bytes(const lcn_model* m, int64_t n_rows, 
   return lcn_ws_layout(m, n_rows, bn_group, training).total;
 }
 
-// prepare only touches the head of the workspace, whose offsets do not depend on the row geometry
-extern "C" int lcn_model_prepare_weights(lcn_model* m, const float* d_params, void* d_ws, size_t ws_bytes, void* stream) {
-  LCN_REQUIRE(m && d_params && d_ws, "null argument");
-  WsLayout lay = lcn_ws_layout(m, 128, 128, 0);
-  if (ws_bytes < lay.off_part) {
-    lcn_set_error("workspace too small: %zu < %zu", ws_bytes, lay.off_part);
+// *lay = the workspace layout of a call; LCN_ENOMEM when ws_bytes is short of it.  head_only: the call touches only the
+// head of the workspace (packed weights, mask, scalars), whose offsets do not depend on the row geometry.
+static int ws_layout_for(const lcn_model* m, int64_t n_rows, int bn_group, int training, size_t ws_bytes,
+                         bool head_only, WsLayout* lay) {
+  *lay = lcn_ws_layout(m, n_rows, bn_group, training);
+  const size_t need = head_only ? lay->off_part : lay->total;
+  if (ws_bytes < need) {
+    lcn_set_error("workspace too small: %zu < %zu", ws_bytes, need);
     return LCN_ENOMEM;
   }
+  return LCN_OK;
+}
+
+extern "C" int lcn_model_prepare_weights(lcn_model* m, const float* d_params, void* d_ws, size_t ws_bytes, void* stream) {
+  LCN_REQUIRE(m && d_params && d_ws, "null argument");
+  WsLayout lay;
+  int rc = ws_layout_for(m, 128, 128, 0, ws_bytes, true, &lay);
+  if (rc) return rc;
   return lcn_launch_prepare(m, d_params, (char*)d_ws, lay, true, (cudaStream_t)stream);
 }
 
@@ -408,22 +406,16 @@ extern "C" int lcn_debug_trace_dump() {
   return n;
 }
 
-extern "C" int lcn_model_forward(lcn_model* m, const float* d_params, void* d_ws, size_t ws_bytes, const float* d_x,
-                                 int64_t n_rows, int32_t bn_group, int training, float dropout_rate, uint64_t seed,
-                                 uint64_t step, float* d_out, const lcn_step_scalars* d_dyn, void* stream) {
-  int rc = check_geom(m, n_rows, bn_group);
-  if (rc) return rc;
-  LCN_REQUIRE(d_params && d_ws && d_x && d_out, "null argument");
-  LCN_REQUIRE(dropout_rate >= 0.f && dropout_rate < 1.f, "dropout rate %f outside [0,1)", dropout_rate);
+// the forward pass of lcn_model_forward / lcn_model_forward_layers once their arguments are checked
+static int run_forward(lcn_model* m, const float* d_params, void* d_ws, size_t ws_bytes, const float* d_x,
+                       int64_t n_rows, int32_t bn_group, int training, float dropout_rate, uint64_t seed, uint64_t step,
+                       float* d_out, const lcn_step_scalars* d_dyn, int layer_begin, int layer_end, void* stream) {
   FwdArgs a;
+  int rc = ws_layout_for(m, n_rows, bn_group, training, ws_bytes, false, &a.lay);
+  if (rc) return rc;
   a.m = m;
   a.params = d_params;
   a.ws = (char*)d_ws;
-  a.lay = lcn_ws_layout(m, n_rows, bn_group, training);
-  if (ws_bytes < a.lay.total) {
-    lcn_set_error("workspace too small: %zu < %zu", ws_bytes, a.lay.total);
-    return LCN_ENOMEM;
-  }
   a.x = d_x;
   a.out = d_out;
   a.dropout_rate = dropout_rate;
@@ -431,7 +423,20 @@ extern "C" int lcn_model_forward(lcn_model* m, const float* d_params, void* d_ws
   a.step = step;
   a.dyn = d_dyn;
   a.st = (cudaStream_t)stream;
+  a.layer_begin = layer_begin;
+  a.layer_end = layer_end;
   return lcn_launch_forward(a);
+}
+
+extern "C" int lcn_model_forward(lcn_model* m, const float* d_params, void* d_ws, size_t ws_bytes, const float* d_x,
+                                 int64_t n_rows, int32_t bn_group, int training, float dropout_rate, uint64_t seed,
+                                 uint64_t step, float* d_out, const lcn_step_scalars* d_dyn, void* stream) {
+  int rc = check_geom(m, n_rows, bn_group);
+  if (rc) return rc;
+  LCN_REQUIRE(d_params && d_ws && d_x && d_out, "null argument");
+  LCN_REQUIRE(dropout_rate >= 0.f && dropout_rate < 1.f, "dropout rate %f outside [0,1)", dropout_rate);
+  return run_forward(m, d_params, d_ws, ws_bytes, d_x, n_rows, bn_group, training, dropout_rate, seed, step, d_out, d_dyn,
+                     0, -1, stream);
 }
 
 extern "C" int lcn_model_forward_layers(lcn_model* m, const float* d_params, void* d_ws, size_t ws_bytes, const float* d_x,
@@ -449,25 +454,9 @@ extern "C" int lcn_model_forward_layers(lcn_model* m, const float* d_params, voi
     lcn_set_error("lcn_model_forward_layers: not available while synchronised BatchNorm is on (lcn_dp_sync_batch_norm)");
     return LCN_ESTATE;
   }
-  FwdArgs a;
-  a.m = m;
-  a.params = d_params;
-  a.ws = (char*)d_ws;
-  a.lay = lcn_ws_layout(m, n_rows, bn_group, 1);     // training layout: every Z_l / A_l has its own buffer
-  if (ws_bytes < a.lay.total) {
-    lcn_set_error("workspace too small: %zu < %zu", ws_bytes, a.lay.total);
-    return LCN_ENOMEM;
-  }
-  a.x = d_x;
-  a.out = d_out;
-  a.dropout_rate = dropout_rate;
-  a.seed = seed;
-  a.step = step;
-  a.dyn = nullptr;
-  a.st = (cudaStream_t)stream;
-  a.layer_begin = layer_begin;
-  a.layer_end = layer_end;
-  return lcn_launch_forward(a);
+  // training layout: every Z_l / A_l has its own buffer
+  return run_forward(m, d_params, d_ws, ws_bytes, d_x, n_rows, bn_group, 1, dropout_rate, seed, step, d_out, nullptr,
+                     layer_begin, layer_end, stream);
 }
 
 extern "C" int lcn_model_write_tensor(lcn_model* m, void* d_ws, size_t ws_bytes, int kind, int layer, int64_t n_rows,
@@ -476,11 +465,9 @@ extern "C" int lcn_model_write_tensor(lcn_model* m, void* d_ws, size_t ws_bytes,
   if (rc) return rc;
   LCN_REQUIRE(d_ws && d_src, "null argument");
   LCN_REQUIRE(kind == 1, "only kind 1 (layer output A_l) can be injected");
-  WsLayout lay = lcn_ws_layout(m, n_rows, bn_group, 1);
-  if (ws_bytes < lay.total) {
-    lcn_set_error("workspace too small: %zu < %zu", ws_bytes, lay.total);
-    return LCN_ENOMEM;
-  }
+  WsLayout lay;
+  rc = ws_layout_for(m, n_rows, bn_group, 1, ws_bytes, false, &lay);
+  if (rc) return rc;
   return lcn_launch_write_tensor(m, (char*)d_ws, lay, layer, d_src, (cudaStream_t)stream);
 }
 
@@ -490,12 +477,10 @@ extern "C" int lcn_model_forward_taps(lcn_model* m, const float* d_params, void*
   int rc = check_geom(m, n_rows, bn_group);
   if (rc) return rc;
   LCN_REQUIRE(d_params && d_ws && d_x && d_out && d_taps, "null argument");
-  WsLayout lay = lcn_ws_layout(m, n_rows, bn_group, 0);
-  LCN_REQUIRE(lay.fused, "forward_taps: the fused inference kernel does not cover this model / bn_group");
-  if (ws_bytes < lay.total) {
-    lcn_set_error("workspace too small: %zu < %zu", ws_bytes, lay.total);
-    return LCN_ENOMEM;
-  }
+  LCN_REQUIRE(lcn_stack_eligible(m, bn_group, 0), "forward_taps: the fused inference kernel does not cover this model / bn_group");
+  WsLayout lay;
+  rc = ws_layout_for(m, n_rows, bn_group, 0, ws_bytes, false, &lay);
+  if (rc) return rc;
   size_t need = (size_t)m->n_bn * lay.tiles * LCN_J * 8192 * 2;
   LCN_REQUIRE(taps_bytes >= need, "taps buffer too small: %zu < %zu", taps_bytes, need);
   return lcn_stack_forward(m, lay, d_params, (char*)d_ws, d_x, d_out, d_taps, (cudaStream_t)stream);
@@ -508,11 +493,9 @@ extern "C" int lcn_model_backward(lcn_model* m, const float* d_params, void* d_w
   int rc = check_geom(m, n_rows, (int32_t)n_rows);
   if (rc) return rc;
   LCN_REQUIRE(d_params && d_ws && d_x && d_labels && d_loss && d_grads_raw, "null argument");
-  WsLayout lay = lcn_ws_layout(m, n_rows, (int)n_rows, 1);   // training: the batch is one BN group
-  if (ws_bytes < lay.total) {
-    lcn_set_error("workspace too small: %zu < %zu", ws_bytes, lay.total);
-    return LCN_ENOMEM;
-  }
+  WsLayout lay;
+  rc = ws_layout_for(m, n_rows, (int)n_rows, 1, ws_bytes, false, &lay);   // training: the batch is one BN group
+  if (rc) return rc;
   return lcn_launch_backward(m, d_params, (char*)d_ws, lay, d_x, d_labels, dropout_rate, seed, step, d_loss,
                              d_grads_raw, (cudaStream_t)stream);
 }
@@ -520,11 +503,9 @@ extern "C" int lcn_model_backward(lcn_model* m, const float* d_params, void* d_w
 extern "C" int lcn_model_finalize_grads(lcn_model* m, const float* d_params, void* d_ws, size_t ws_bytes,
                                         const float* d_grads_raw, float* d_grads_out, void* stream) {
   LCN_REQUIRE(m && d_params && d_ws && d_grads_raw && d_grads_out, "null argument");
-  WsLayout lay = lcn_ws_layout(m, 128, 128, 0);
-  if (ws_bytes < lay.off_part) {
-    lcn_set_error("workspace too small");
-    return LCN_ENOMEM;
-  }
+  WsLayout lay;
+  int rc = ws_layout_for(m, 128, 128, 0, ws_bytes, true, &lay);
+  if (rc) return rc;
   return lcn_launch_grad_finalize(m, d_params, (char*)d_ws, lay, d_grads_raw, d_grads_out, (cudaStream_t)stream);
 }
 
@@ -532,11 +513,9 @@ extern "C" int lcn_model_adam_step(lcn_model* m, float* d_params, float* d_m, fl
                                    const float* d_grads_raw, float lr_t, float beta1, float beta2, float eps,
                                    float regularization, const lcn_step_scalars* d_dyn, void* stream) {
   LCN_REQUIRE(m && d_params && d_m && d_v && d_ws && d_grads_raw, "null argument");
-  WsLayout lay = lcn_ws_layout(m, 128, 128, 0);
-  if (ws_bytes < lay.off_part) {
-    lcn_set_error("workspace too small");
-    return LCN_ENOMEM;
-  }
+  WsLayout lay;
+  int rc = ws_layout_for(m, 128, 128, 0, ws_bytes, true, &lay);
+  if (rc) return rc;
   return lcn_launch_adam(m, d_params, d_m, d_v, (char*)d_ws, lay, d_grads_raw, lr_t, beta1, beta2, eps, regularization,
                          d_dyn, (cudaStream_t)stream);
 }
@@ -557,11 +536,9 @@ extern "C" int lcn_layer_gemm(lcn_model* m, const float* d_params, void* d_ws, s
   if (rc) return rc;
   LCN_REQUIRE(d_params && d_ws, "null argument");
   LCN_REQUIRE(layer >= 1 && layer <= 2 * m->d.num_layers, "layer %d is not a mid layer", layer);
-  WsLayout lay = lcn_ws_layout(m, n_rows, bn_group, 1);
-  if (ws_bytes < lay.total) {
-    lcn_set_error("workspace too small: %zu < %zu", ws_bytes, lay.total);
-    return LCN_ENOMEM;
-  }
+  WsLayout lay;
+  rc = ws_layout_for(m, n_rows, bn_group, 1, ws_bytes, false, &lay);
+  if (rc) return rc;
   return lcn_launch_layer_gemm(m, d_params, (char*)d_ws, lay, layer, transposed, (cudaStream_t)stream);
 }
 
@@ -570,11 +547,8 @@ extern "C" int lcn_model_read_tensor(lcn_model* m, void* d_ws, size_t ws_bytes, 
   int rc = check_geom(m, n_rows, bn_group);
   if (rc) return rc;
   LCN_REQUIRE(d_ws && d_dst, "null argument");
-  WsLayout lay = lcn_ws_layout(m, n_rows, bn_group, 1);
-  size_t need = (kind == 2 || kind == 3) ? lay.off_part : lay.total;   // weights / mask live in the head
-  if (ws_bytes < need) {
-    lcn_set_error("workspace too small: %zu < %zu", ws_bytes, need);
-    return LCN_ENOMEM;
-  }
+  WsLayout lay;
+  rc = ws_layout_for(m, n_rows, bn_group, 1, ws_bytes, kind == 2 || kind == 3, &lay);   // weights / mask live in the head
+  if (rc) return rc;
   return lcn_launch_read_tensor(m, (char*)d_ws, lay, kind, layer, d_dst, (cudaStream_t)stream);
 }

@@ -63,19 +63,22 @@ struct TensorMeta {
   int rows, cols;
 };
 
-// Side stream of the backward pass (bf16 tensor-core path): the weight-gradient GEMM of layer l is off the critical
-// path (dZ_l -> dgrad_l -> BN backward of l-1 -> ...), so it is enqueued on a stream owned by the model and joined
-// with events (plain fork/join, capturable into the caller's CUDA graph).  Created on first use; `mu` serialises
-// the enqueue of concurrent backward calls on the same model (the events are shared).
+// Side streams of the model.  The weight-gradient GEMM of layer l is off the critical path of the backward pass
+// (dZ_l -> dgrad_l -> BN backward of l-1 -> ...), so it is enqueued on a stream owned by the model and joined with
+// events (plain fork/join, capturable into the caller's CUDA graph); the weight preparation packs the edge layers
+// there too.  Created on first use (lcn_kernels.cu); `mu` serialises the enqueue of concurrent calls on the same model
+// (the events are shared).
 struct LcnAux {
   std::mutex mu;
-  bool ready = false, failed = false;
+  bool ready = false;
   cudaStream_t st = nullptr;
   cudaStream_t xst = nullptr;        // data-parallel exchange of finished weight gradients (lcn_dp.cu), forked from `st`
   cudaEvent_t ev_xdone = nullptr;
   cudaEvent_t ev_go = nullptr, ev_done = nullptr, ev_ms = nullptr, ev_loss = nullptr;
   cudaEvent_t ev_dz[2] = {nullptr, nullptr}, ev_wg[2] = {nullptr, nullptr};
 };
+
+void lcn_aux_release(LcnAux& a);   // destroys the streams and events created so far
 
 struct LcnDp;                      // data-parallel exchange buffers mapped across the ranks (lcn_dp.cu); null: single process
 

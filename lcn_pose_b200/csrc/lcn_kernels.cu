@@ -309,24 +309,44 @@ __global__ void __launch_bounds__(256) k_pack_edges(const float* __restrict__ pa
   }
 }
 
-// side stream + events of the model (LcnAux), created on first use under aux.mu (held by the caller); nullptr when
-// the creation failed -- the callers then enqueue everything on the caller's stream
-static LcnAux* lcn_aux_get(const lcn_model* m) {
+// side stream + events of the model (LcnAux), created on first use under aux.mu (held by the caller).  A creation that
+// fails releases what was created and returns LCN_ECUDA; the next call tries again.
+void lcn_aux_release(LcnAux& a) {
+  for (cudaStream_t* s : {&a.st, &a.xst}) {
+    if (*s != nullptr) cudaStreamDestroy(*s);
+    *s = nullptr;
+  }
+  for (cudaEvent_t* e : {&a.ev_go, &a.ev_done, &a.ev_dz[0], &a.ev_dz[1], &a.ev_wg[0], &a.ev_wg[1], &a.ev_ms, &a.ev_loss,
+                         &a.ev_xdone}) {
+    if (*e != nullptr) cudaEventDestroy(*e);
+    *e = nullptr;
+  }
+  a.ready = false;
+}
+
+static int lcn_aux_get(const lcn_model* m, LcnAux** out) {
   LcnAux& a = m->aux;
-  if (a.failed) return nullptr;
   if (!a.ready) {
-    bool ok = cudaStreamCreateWithFlags(&a.st, cudaStreamNonBlocking) == cudaSuccess;
-    ok = ok && cudaStreamCreateWithFlags(&a.xst, cudaStreamNonBlocking) == cudaSuccess;
-    cudaEvent_t* evs[9] = {&a.ev_go, &a.ev_done, &a.ev_dz[0], &a.ev_dz[1], &a.ev_wg[0], &a.ev_wg[1], &a.ev_ms, &a.ev_loss, &a.ev_xdone};
-    for (int i = 0; i < 9 && ok; ++i) ok = cudaEventCreateWithFlags(evs[i], cudaEventDisableTiming) == cudaSuccess;
-    if (!ok) {
+    const char* call = "cudaStreamCreateWithFlags";
+    cudaError_t e = cudaSuccess;
+    for (cudaStream_t* s : {&a.st, &a.xst})
+      if (e == cudaSuccess) e = cudaStreamCreateWithFlags(s, cudaStreamNonBlocking);
+    if (e == cudaSuccess) {
+      call = "cudaEventCreateWithFlags";
+      for (cudaEvent_t* ev : {&a.ev_go, &a.ev_done, &a.ev_dz[0], &a.ev_dz[1], &a.ev_wg[0], &a.ev_wg[1], &a.ev_ms,
+                              &a.ev_loss, &a.ev_xdone})
+        if (e == cudaSuccess) e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
+    }
+    if (e != cudaSuccess) {
       (void)cudaGetLastError();
-      a.failed = true;
-      return nullptr;
+      lcn_aux_release(a);
+      lcn_set_error("side streams of the model: %s -> %s", call, cudaGetErrorString(e));
+      return LCN_ECUDA;
     }
     a.ready = true;
   }
-  return &a;
+  *out = &a;
+  return LCN_OK;
 }
 
 int lcn_launch_prepare(const lcn_model* m, const float* params, char* ws, const WsLayout& lay,
@@ -345,62 +365,50 @@ int lcn_launch_prepare(const lcn_model* m, const float* params, char* ws, const 
   int n_mid = m->n_lin - 2;
   const bool x3 = m->d.path == LCN_PATH_FP32;
   const bool bf = m->d.path == LCN_PATH_BF16;
-  // With mid layers and a first layer of <= 64 input features (every configuration of the reference) the weight
-  // preparation is two concurrent launches: k_pack_mid on the caller's stream (it also stores the mask values and the
-  // per-layer scalars for the kernels that follow) and k_pack_edges on the model's side stream.  Otherwise the general
-  // sequence k_mask_scalars -> k_pack_edge (-> bf16 tiles) per edge layer.
-  const bool fused_prep = n_mid > 0 && m->L[0].Kin <= 64;
-  if (!fused_prep) {
+  if (n_mid == 0) {
+    // no mid layers: k_mask_scalars, then each edge layer (-> bf16 tiles), in order on the caller's stream
     lcn_launch(k_mask_scalars, dim3(1), dim3(320), 0, st, params, m->mask_off, m->sup, cmask, m->n_lin, m->d.max_norm, sc, mask);
     LCN_CHECK_LAUNCH();
-  }
-  std::unique_lock<std::mutex> aux_lock;
-  LcnAux* ax = nullptr;
-  if (n_mid > 0) {
-    aux_lock = std::unique_lock<std::mutex>(m->aux.mu);
-    ax = lcn_aux_get(m);
-    if (ax == nullptr) aux_lock.unlock();
-  }
-  cudaStream_t est = ax ? ax->st : st;
-  if (ax) {
-    LCN_CHECK_CUDA(cudaEventRecord(ax->ev_go, st));
-    LCN_CHECK_CUDA(cudaStreamWaitEvent(est, ax->ev_go, 0));
-  }
-  if (fused_prep) {
-    lcn_launch(k_pack_edges, dim3(LCN_J * m->FC, 4, 2), dim3(256), 0, est, params, m->L[0].w_off, m->L[last].w_off, m->d.in_F,
-               m->d.F, m->P, last, static_cast<const LayerScalars*>(sc), m->mask_off, cmask, m->sup, m->d.max_norm,
-               reinterpret_cast<float*>(ws + lay.off_wm_first), reinterpret_cast<float*>(ws + lay.off_wm_last),
-               bf ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wf16) : nullptr,
-               bf ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wl16f) : nullptr,
-               bf ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wl16b) : nullptr);
-  } else {
-    lcn_launch(k_pack_edge, dim3(64), dim3(256), 0, est, params + m->L[0].w_off, m->L[0].Fi, m->L[0].Fo, sc, 0, mask,
+    lcn_launch(k_pack_edge, dim3(64), dim3(256), 0, st, params + m->L[0].w_off, m->L[0].Fi, m->L[0].Fo, sc, 0, mask,
                                     reinterpret_cast<float*>(ws + lay.off_wm_first));
-    if (bf && m->L[0].Kin <= 64)
-      lcn_launch(k_pack_first16, dim3(LCN_J * m->FC, 4), dim3(256), 0, est, reinterpret_cast<const float*>(ws + lay.off_wm_first), m->L[0].Kin,
+    if (bf)
+      lcn_launch(k_pack_first16, dim3(LCN_J * m->FC, 4), dim3(256), 0, st, reinterpret_cast<const float*>(ws + lay.off_wm_first), m->L[0].Kin,
                                                     m->P, reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wf16));
-  }
-  if (ax) LCN_CHECK_CUDA(cudaEventRecord(ax->ev_done, est));
-  if (n_mid > 0) {
-    lcn_launch(k_pack_mid, dim3(dim3(m->nnz * m->FC * m->FC, n_mid)), dim3(256), 0, st, 
-        params, lt, make_pairs(m), m->sup, sc, mask, m->d.F, m->FC, m->nnz,
-        reinterpret_cast<float*>(ws + lay.off_wp32), reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16f),
-        reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16b),
-        x3 ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16f_lo) : nullptr,
-        x3 ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16b_lo) : nullptr,
-        x3 ? 1 : 0 /* fp32 copy: the parity tap of the fp32-parity path (lcn_model_read_tensor kind 2) */, 1,
-        m->mask_off, cmask, m->n_lin, m->d.max_norm, fused_prep ? sc : nullptr, fused_prep ? mask : nullptr);
-  }
-  if (!fused_prep) {
     lcn_launch(k_pack_edge, dim3(64), dim3(256), 0, st, params + m->L[last].w_off, m->L[last].Fi, m->L[last].Fo, sc, last, mask,
                                     reinterpret_cast<float*>(ws + lay.off_wm_last));
     if (bf)
       lcn_launch(k_pack_last16, dim3(LCN_J * m->FC, 4), dim3(256), 0, st, reinterpret_cast<const float*>(ws + lay.off_wm_last),
                                                    reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wl16f),
                                                    reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wl16b));
+    LCN_CHECK_LAUNCH();
+    return LCN_OK;
   }
+  // With mid layers the weight preparation is two concurrent launches: k_pack_mid on the caller's stream (it also
+  // stores the mask values and the per-layer scalars for the kernels that follow) and k_pack_edges on the model's side
+  // stream.
+  std::lock_guard<std::mutex> aux_lock(m->aux.mu);
+  LcnAux* ax;
+  int rc = lcn_aux_get(m, &ax);
+  if (rc) return rc;
+  LCN_CHECK_CUDA(cudaEventRecord(ax->ev_go, st));
+  LCN_CHECK_CUDA(cudaStreamWaitEvent(ax->st, ax->ev_go, 0));
+  lcn_launch(k_pack_edges, dim3(LCN_J * m->FC, 4, 2), dim3(256), 0, ax->st, params, m->L[0].w_off, m->L[last].w_off, m->d.in_F,
+             m->d.F, m->P, last, static_cast<const LayerScalars*>(sc), m->mask_off, cmask, m->sup, m->d.max_norm,
+             reinterpret_cast<float*>(ws + lay.off_wm_first), reinterpret_cast<float*>(ws + lay.off_wm_last),
+             bf ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wf16) : nullptr,
+             bf ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wl16f) : nullptr,
+             bf ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wl16b) : nullptr);
+  LCN_CHECK_CUDA(cudaEventRecord(ax->ev_done, ax->st));
+  lcn_launch(k_pack_mid, dim3(dim3(m->nnz * m->FC * m->FC, n_mid)), dim3(256), 0, st, 
+      params, lt, make_pairs(m), m->sup, sc, mask, m->d.F, m->FC, m->nnz,
+      reinterpret_cast<float*>(ws + lay.off_wp32), reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16f),
+      reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16b),
+      x3 ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16f_lo) : nullptr,
+      x3 ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16b_lo) : nullptr,
+      x3 ? 1 : 0 /* fp32 copy: the parity tap of the fp32-parity path (lcn_model_read_tensor kind 2) */, 1,
+      m->mask_off, cmask, m->n_lin, m->d.max_norm, sc, mask);
   LCN_CHECK_LAUNCH();
-  if (ax) LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_done, 0));
+  LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_done, 0));
   return LCN_OK;
 }
 
@@ -1767,6 +1775,27 @@ static inline char* a_buf(char* ws, const WsLayout& lay, int l) {
 static inline float* bn_stat(char* ws, const WsLayout& lay, const lcn_model* m, int l) {
   return reinterpret_cast<float*>(ws + lay.off_bnstat) + (size_t)l * lay.n_groups * m->d.F * 2;
 }
+// launch geometry of the elementwise BatchNorm kernels (k_bn_act*, k_bn_bwd_*): blocks of (P/8, ewy) threads over
+// grid-stride row ranges of rows_thr rows per thread
+struct EwGeom {
+  int ewy, grid, rows_thr;
+};
+static inline EwGeom ew_geom(const lcn_model* m, const WsLayout& lay) {
+  const int ewy = (m->P / 8) * 2 <= EW_MAXT ? 2 : 1;
+  const int grid = (int)std::min<int64_t>(2 * m->sm_count, lay.rows_pad / ewy);
+  return {ewy, grid, (int)((lay.rows_pad / ewy + grid - 1) / grid)};
+}
+// packed bf16 blocks of mid layer l: forward (Y = A*Wm) or transposed (dA = dZ*Wm^T); lo: their lo parts on the
+// split-bf16 path, nullptr on the bf16 path
+struct MidWeights {
+  const char *hi, *lo;
+};
+static inline MidWeights mid_weights(const lcn_model* m, const char* ws, const WsLayout& lay, int l, int transposed) {
+  const size_t ofs = (size_t)(l - 1) * m->nnz * m->FC * m->FC * 4096 * 2;
+  const bool x3 = m->d.path == LCN_PATH_FP32;
+  return {ws + (transposed ? lay.off_wp16b : lay.off_wp16f) + ofs,
+          x3 ? ws + (transposed ? lay.off_wp16b_lo : lay.off_wp16f_lo) + ofs : nullptr};
+}
 
 template <typename T>
 static int forward_impl(const FwdArgs& a) {
@@ -1777,7 +1806,7 @@ static int forward_impl(const FwdArgs& a) {
   const int P = m->P, F = m->d.F, FC = m->FC;
   RowGeom g{lay.n_rows, lay.bn_group, lay.gstride};
   float* part = reinterpret_cast<float*>(ws + lay.off_part);
-  constexpr bool kBf = PathTraits<T>::bf16, kX3 = PathTraits<T>::x3;
+  constexpr bool kBf = PathTraits<T>::bf16;
   size_t gemm_smem = (LCN_TILE * GS_APAD + 64 * GS_BPAD) * sizeof(float);
   static std::once_flag attr_once;                 // one per instantiation; thread safe (header: re-entrancy)
   static cudaError_t attr_rc = cudaSuccess;
@@ -1786,16 +1815,12 @@ static int forward_impl(const FwdArgs& a) {
   });
   LCN_CHECK_CUDA(attr_rc);
   int n_bn = m->n_bn;
-  // training at one BatchNorm group on the tensor-core path: the mid-layer GEMMs accumulate the BatchNorm statistics
-  // themselves (TcFuse, lcn_gemm_tc.cu) and k_bn_act_pre finalises them; the accumulators are cleared here, once per pass
-  bool pre_ok = false;                 // k_bn_act_pre eligible (same test as below): it is the kernel that accepts gacc
-  if constexpr (kBf) {
-    const int ewy0 = (P / 8) * 2 <= EW_MAXT ? 2 : 1;
-    const int grid0 = (int)std::min<int64_t>(2 * m->sm_count, lay.rows_pad / ewy0);
-    const int per0 = (int)(((lay.rows_pad / ewy0 + grid0 - 1) / grid0) * ewy0);
-    pre_ok = lay.n_groups == 1 && per0 <= BA_R * ewy0;
-  }
-  const bool try_fuse = kBf && lay.training && lay.n_groups == 1 && pre_ok;
+  const EwGeom ew = ew_geom(m, lay);
+  // k_bn_act_pre takes every layer on the bf16 path at one BatchNorm group and <= BA_R rows per thread (all loads up
+  // front).  In training the mid-layer GEMMs then accumulate the BatchNorm statistics themselves (TcFuse,
+  // lcn_gemm_tc.cu) and k_bn_act_pre finalises them; the accumulators are cleared here, once per pass
+  const bool pre = kBf && lay.n_groups == 1 && ew.rows_thr <= BA_R;
+  const bool try_fuse = pre && lay.training;
   const bool bn_sync = lay.training && lcn_bn_sync_on(m);      // lcn_model_forward admits it only at one group
   if (bn_sync && lay.n_groups != 1) {
     lcn_set_error("synchronised BatchNorm: a training forward pass must be one BatchNorm group (bn_group = n_rows)");
@@ -1821,16 +1846,16 @@ static int forward_impl(const FwdArgs& a) {
       }
     } else {
       const T* Ain = reinterpret_cast<const T*>(a_buf(ws, lay, l - 1));
-      const size_t wofs = (size_t)(l - 1) * m->nnz * FC * FC * 4096 * 2;
+      const MidWeights w = mid_weights(m, ws, lay, l, 0);
       TcFuse fu;
       memset(&fu, 0, sizeof(fu));
       if (try_fuse) {
         fu.gacc = reinterpret_cast<double*>(ws + lay.off_gacc + (size_t)l * lay.gacc_stride);
         fu.F = F;
       }
-      int rc = lcn_tc_gemm(m, lay, l - 1, 0, reinterpret_cast<const __nv_bfloat16*>(Ain), ws + lay.off_wp16f + wofs,
-                           a.params + L.b_off, nullptr, reinterpret_cast<__nv_bfloat16*>(Z), part, st,
-                           try_fuse ? &fu : nullptr, &fused_bn, kX3 ? ws + lay.off_wp16f_lo + wofs : nullptr);
+      int rc = lcn_tc_gemm(m, lay, l - 1, 0, reinterpret_cast<const __nv_bfloat16*>(Ain), w.hi, a.params + L.b_off,
+                           nullptr, reinterpret_cast<__nv_bfloat16*>(Z), part, st, try_fuse ? &fu : nullptr, &fused_bn,
+                           w.lo);
       if (rc) return rc;
     }
     LCN_CHECK_LAUNCH();
@@ -1849,29 +1874,16 @@ static int forward_impl(const FwdArgs& a) {
       gacc = nullptr;                  // k_bn_act_pre reads the global statistics from stat
     }
     const T* res = L.res_from >= 0 ? reinterpret_cast<const T*>(a_buf(ws, lay, L.res_from)) : nullptr;
-    const int ewy = (P / 8) * 2 <= EW_MAXT ? 2 : 1;
     uint8_t* keepbits = (lay.training && a.dropout_rate > 0.f)
                             ? reinterpret_cast<uint8_t*>(ws + lay.off_keep) + (size_t)l * lay.rows_pad * (P / 8)
                             : nullptr;
-    int ew_grid = (int)std::min<int64_t>(2 * m->sm_count, lay.rows_pad / ewy);
-    bool pre = false;
-    if constexpr (kBf) {
-      // one BN group, <= BA_R rows per thread: all loads up front (k_bn_act_pre)
-      const int per = (int)(((lay.rows_pad / ewy + ew_grid - 1) / ew_grid) * ewy);
-      if (lay.n_groups == 1 && per <= BA_R * ewy) {
-        pre = true;
-        lcn_launch(k_bn_act_pre, dim3(ew_grid), dim3(P / 8, ewy), 0, st, reinterpret_cast<const __nv_bfloat16*>(Z), stat,
-                   a.params + L.gamma_off, a.params + L.beta_off, reinterpret_cast<const __nv_bfloat16*>(res),
-                   reinterpret_cast<__nv_bfloat16*>(Aout), keepbits, P, F, (int)lay.rows_pad, lay.bn_group, a.dropout_rate,
-                   a.seed, a.step, l, a.dyn, gacc, stat, 1.0 / ((double)lay.bn_group * LCN_J));
-      }
-    }
-    if (!pre && fused_bn) {
-      lcn_set_error("internal: BatchNorm statistics were accumulated for k_bn_act_pre, which is not eligible here");
-      return LCN_EINVAL;
-    }
-    if (!pre)
-      lcn_launch(k_bn_act<T>, dim3(ew_grid), dim3(dim3(P / 8, ewy)), 0, st, Z, stat, a.params + L.gamma_off, a.params + L.beta_off, res, Aout,
+    if (pre)
+      lcn_launch(k_bn_act_pre, dim3(ew.grid), dim3(P / 8, ew.ewy), 0, st, reinterpret_cast<const __nv_bfloat16*>(Z), stat,
+                 a.params + L.gamma_off, a.params + L.beta_off, reinterpret_cast<const __nv_bfloat16*>(res),
+                 reinterpret_cast<__nv_bfloat16*>(Aout), keepbits, P, F, (int)lay.rows_pad, lay.bn_group, a.dropout_rate,
+                 a.seed, a.step, l, a.dyn, gacc, stat, 1.0 / ((double)lay.bn_group * LCN_J));
+    else
+      lcn_launch(k_bn_act<T>, dim3(ew.grid), dim3(dim3(P / 8, ew.ewy)), 0, st, Z, stat, a.params + L.gamma_off, a.params + L.beta_off, res, Aout,
                                                       keepbits, P, F, (int)lay.rows_pad, lay.bn_group, lay.gstride,
                                                       a.dropout_rate, a.seed, a.step, l, a.dyn);
     LCN_CHECK_LAUNCH();
@@ -1908,37 +1920,33 @@ template <typename T>
 static int backward_impl(const lcn_model* m, const float* params, char* ws, const WsLayout& lay, const float* x,
                          const float* labels, float rate, uint64_t seed, uint64_t step, float* loss,
                          float* graw, cudaStream_t st) {
-  const int P = m->P, F = m->d.F, FC = m->FC;
+  const int P = m->P, F = m->d.F;
   constexpr bool kBf = PathTraits<T>::bf16, kX3 = PathTraits<T>::x3;
   // weight-gradient GEMMs go to the model's side stream (see LcnAux); `wst` is the stream they are enqueued on
-  std::unique_lock<std::mutex> aux_lock(m->aux.mu);
-  LcnAux* ax = lcn_aux_get(m);
-  if (ax == nullptr) aux_lock.unlock();
-  cudaStream_t wst = ax ? ax->st : st;
-  // data parallel (lcn_dp.cu): with a side stream the mean of every mid-layer weight gradient is exchanged over NVLink on a
-  // third stream as soon as its GEMM has finished, under the rest of the backward pass; what is left for the end is the
+  std::lock_guard<std::mutex> aux_lock(m->aux.mu);
+  LcnAux* ax;
+  int rc = lcn_aux_get(m, &ax);
+  if (rc) return rc;
+  cudaStream_t wst = ax->st;
+  // data parallel (lcn_dp.cu): in mode 1 the mean of every mid-layer weight gradient is exchanged over NVLink on a third
+  // stream as soon as its GEMM has finished, under the rest of the backward pass; what is left for the end is the
   // first and last layer and the small tensors (< 2 % of the bucket)
   const int dp_mode = lcn_dp_mode(m);
-  const bool dp_stream = dp_mode == 1 && ax != nullptr;
   const bool bn_sync = lcn_bn_sync_on(m);
   bool dp_forked = false;
   bool wg_pending[2] = {false, false};
   const int64_t blast = m->L[m->n_lin - 1].b_off;     // last-layer bias gradient: accumulated by k_loss_dout (caller's stream)
-  if (ax) {
-    // fork at the very start: the 4 B/parameter clear of the gradient bucket (the weight-gradient GEMMs reduce-add
-    // into it) leaves the critical path; the caller's stream only clears what its own first kernels accumulate into
-    LCN_CHECK_CUDA(cudaEventRecord(ax->ev_go, st));
-    LCN_CHECK_CUDA(cudaStreamWaitEvent(wst, ax->ev_go, 0));
-    LCN_CHECK_CUDA(cudaMemsetAsync(graw, 0, sizeof(float) * blast, wst));
-    if (blast + 51 < m->n_params)
-      LCN_CHECK_CUDA(cudaMemsetAsync(graw + blast + 51, 0, sizeof(float) * (m->n_params - blast - 51), wst));
-    LCN_CHECK_CUDA(cudaMemsetAsync(ws + lay.off_dw_last, 0, sizeof(float) * P * 64, wst));
-    LCN_CHECK_CUDA(cudaMemsetAsync(ws + lay.off_dw_first, 0, sizeof(float) * 64 * P, wst));
-    LCN_CHECK_CUDA(cudaEventRecord(ax->ev_ms, wst));
-    LCN_CHECK_CUDA(cudaMemsetAsync(graw + blast, 0, sizeof(float) * 51, st));
-  } else {
-    LCN_CHECK_CUDA(cudaMemsetAsync(graw, 0, sizeof(float) * m->n_params, st));
-  }
+  // fork at the very start: the 4 B/parameter clear of the gradient bucket (the weight-gradient GEMMs reduce-add
+  // into it) leaves the critical path; the caller's stream only clears what its own first kernels accumulate into
+  LCN_CHECK_CUDA(cudaEventRecord(ax->ev_go, st));
+  LCN_CHECK_CUDA(cudaStreamWaitEvent(wst, ax->ev_go, 0));
+  LCN_CHECK_CUDA(cudaMemsetAsync(graw, 0, sizeof(float) * blast, wst));
+  if (blast + 51 < m->n_params)
+    LCN_CHECK_CUDA(cudaMemsetAsync(graw + blast + 51, 0, sizeof(float) * (m->n_params - blast - 51), wst));
+  LCN_CHECK_CUDA(cudaMemsetAsync(ws + lay.off_dw_last, 0, sizeof(float) * P * 64, wst));
+  LCN_CHECK_CUDA(cudaMemsetAsync(ws + lay.off_dw_first, 0, sizeof(float) * 64 * P, wst));
+  LCN_CHECK_CUDA(cudaEventRecord(ax->ev_ms, wst));
+  LCN_CHECK_CUDA(cudaMemsetAsync(graw + blast, 0, sizeof(float) * 51, st));
   LCN_CHECK_CUDA(cudaMemsetAsync(ws + lay.off_loss, 0, 2 * sizeof(double), st));
   LCN_CHECK_CUDA(cudaMemsetAsync(ws + lay.off_bnsum, 0, sizeof(float) * m->n_bn * (F * 2 + 1), st));   // sums + grid-barrier counters
   float* dout = reinterpret_cast<float*>(ws + lay.off_dout);
@@ -1958,14 +1966,10 @@ static int backward_impl(const lcn_model* m, const float* params, char* ws, cons
   if constexpr (kBf) {
     const __nv_bfloat16* Ain = reinterpret_cast<const __nv_bfloat16*>(a_buf(ws, lay, m->n_bn - 1));
     float* dwl = reinterpret_cast<float*>(ws + lay.off_dw_last);
-    if (ax) {                       // the loss gradient (caller's stream) precedes the last layer's weight gradient
-      LCN_CHECK_CUDA(cudaEventRecord(ax->ev_loss, st));
-      LCN_CHECK_CUDA(cudaStreamWaitEvent(wst, ax->ev_loss, 0));
-    } else {
-      LCN_CHECK_CUDA(cudaMemsetAsync(dwl, 0, sizeof(float) * P * 64, st));
-      LCN_CHECK_CUDA(cudaMemsetAsync(ws + lay.off_dw_first, 0, sizeof(float) * 64 * P, st));
-    }
-    int rc = lcn_tc_head_dgrad(m, lay, dout16, ws + lay.off_wl16b, reinterpret_cast<__nv_bfloat16*>(D(cur)), st);
+    // the loss gradient (caller's stream) precedes the last layer's weight gradient
+    LCN_CHECK_CUDA(cudaEventRecord(ax->ev_loss, st));
+    LCN_CHECK_CUDA(cudaStreamWaitEvent(wst, ax->ev_loss, 0));
+    rc = lcn_tc_head_dgrad(m, lay, dout16, ws + lay.off_wl16b, reinterpret_cast<__nv_bfloat16*>(D(cur)), st);
     if (rc) return rc;
     rc = lcn_tc_wgrad_last(m, lay, Ain, dout16, dwl, wst);
     if (rc) return rc;
@@ -1974,18 +1978,16 @@ static int backward_impl(const lcn_model* m, const float* params, char* ws, cons
   } else {
     // fp32-parity path: the N = 51 head on CUDA cores.  It accumulates dWm4 / db4 with atomics into the bucket, which the
     // side stream is clearing: wait for that first
-    if (ax) LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_ms, 0));
+    LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_ms, 0));
     const T* Ain = reinterpret_cast<const T*>(a_buf(ws, lay, m->n_bn - 1));
     lcn_launch(k_last_layer_bwd<T>, dim3(dim3((unsigned)(lay.rows_pad / rows_blk), (P + 255) / 256)), dim3(256), 0, st, 
         Ain, dout, reinterpret_cast<const float*>(ws + lay.off_wm_last), D(cur), graw + m->L[last].w_off,
         graw + m->L[last].b_off, P, rows_blk);
     LCN_CHECK_LAUNCH();
   }
-  const int ewy = (P / 8) * 2 <= EW_MAXT ? 2 : 1;
-  unsigned eg = (unsigned)std::min<int64_t>(2 * m->sm_count, lay.rows_pad / ewy);
-  size_t red_smem = (size_t)ewy * (P / 8) * 16 * sizeof(float);
-  PairTable pt = make_pairs(m);
-  if (ax) LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_ms, 0));   // the bucket is clear before this stream stores into it
+  const EwGeom ew = ew_geom(m, lay);
+  size_t red_smem = (size_t)ew.ewy * (P / 8) * 16 * sizeof(float);
+  LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_ms, 0));   // the bucket is clear before this stream stores into it
   for (int l = m->n_bn - 1; l >= 0; --l) {
     const LayerInfo& L = m->L[l];
     const T* Z = reinterpret_cast<const T*>(z_buf(ws, lay, l));
@@ -1993,34 +1995,31 @@ static int backward_impl(const lcn_model* m, const float* params, char* ws, cons
     float* sums = reinterpret_cast<float*>(ws + lay.off_bnsum) + (size_t)l * F * 2;
     const uint8_t* keepbits = reinterpret_cast<const uint8_t*>(ws + lay.off_keep) + (size_t)l * lay.rows_pad * (P / 8);
     T* dZ = dZbuf(l);
-    if (ax && wg_pending[l & 1]) {   // the weight gradient of layer l+2 has read this dZ buffer
+    if (wg_pending[l & 1]) {         // the weight gradient of layer l+2 has read this dZ buffer
       LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_wg[l & 1], 0));
       wg_pending[l & 1] = false;
     }
-    {
-      lcn_launch(k_bn_bwd_reduce<T>, dim3(eg), dim3(dim3(P / 8, ewy)), red_smem, st, D(cur), Z, keepbits, stat, params + L.gamma_off,
-                                                               params + L.beta_off, sums, P, F, lay.bn_group, rate);
-      float* gmean = nullptr;          // synchronised BatchNorm: (S1, S2) / N of all ranks, in the layer's accumulator area
-      if (bn_sync) {
-        LCN_CHECK_LAUNCH();
-        gmean = reinterpret_cast<float*>(ws + lay.off_gacc + (size_t)l * lay.gacc_stride);
-        int rc = lcn_bn_sync(m, m->n_bn + l, LCN_BN_SYNC_SUMS, sums, gmean, lay.n_rows, st);
-        if (rc) return rc;
-      }
-      lcn_launch(bn_sync ? k_bn_bwd_apply<T, true> : k_bn_bwd_apply<T, false>, dim3(eg), dim3(dim3(P / 8, ewy)), (size_t)ewy * P * sizeof(float), st,
-          D(cur), Z, keepbits, stat, params + L.gamma_off, params + L.beta_off, sums, dZ,
-          reinterpret_cast<float*>(ws + lay.off_dbpart) + (size_t)l * eg * P, graw + L.gamma_off, graw + L.beta_off, P, F, (int)lay.rows_pad, lay.bn_group, rate,
-          gmean);
+    lcn_launch(k_bn_bwd_reduce<T>, dim3(ew.grid), dim3(dim3(P / 8, ew.ewy)), red_smem, st, D(cur), Z, keepbits, stat, params + L.gamma_off,
+                                                             params + L.beta_off, sums, P, F, lay.bn_group, rate);
+    float* gmean = nullptr;            // synchronised BatchNorm: (S1, S2) / N of all ranks, in the layer's accumulator area
+    if (bn_sync) {
+      LCN_CHECK_LAUNCH();
+      gmean = reinterpret_cast<float*>(ws + lay.off_gacc + (size_t)l * lay.gacc_stride);
+      rc = lcn_bn_sync(m, m->n_bn + l, LCN_BN_SYNC_SUMS, sums, gmean, lay.n_rows, st);
+      if (rc) return rc;
     }
+    lcn_launch(bn_sync ? k_bn_bwd_apply<T, true> : k_bn_bwd_apply<T, false>, dim3(ew.grid), dim3(dim3(P / 8, ew.ewy)), (size_t)ew.ewy * P * sizeof(float), st,
+        D(cur), Z, keepbits, stat, params + L.gamma_off, params + L.beta_off, sums, dZ,
+        reinterpret_cast<float*>(ws + lay.off_dbpart) + (size_t)l * ew.grid * P, graw + L.gamma_off, graw + L.beta_off, P, F, (int)lay.rows_pad, lay.bn_group, rate,
+        gmean);
     LCN_CHECK_LAUNCH();
-    if (ax) {                        // dZ_l is ready: the side stream may start the weight gradient of layer l
-      LCN_CHECK_CUDA(cudaEventRecord(ax->ev_dz[l & 1], st));
-      LCN_CHECK_CUDA(cudaStreamWaitEvent(wst, ax->ev_dz[l & 1], 0));
-    }
+    // dZ_l is ready: the side stream may start the weight gradient of layer l
+    LCN_CHECK_CUDA(cudaEventRecord(ax->ev_dz[l & 1], st));
+    LCN_CHECK_CUDA(cudaStreamWaitEvent(wst, ax->ev_dz[l & 1], 0));
     if (l == 0 && kBf) {
       float* dwf = reinterpret_cast<float*>(ws + lay.off_dw_first);
-      int rc = lcn_tc_wgrad_first(m, lay, reinterpret_cast<const __nv_bfloat16*>(ws + lay.off_x16),
-                                  reinterpret_cast<const __nv_bfloat16*>(dZ), dwf, wst);
+      rc = lcn_tc_wgrad_first(m, lay, reinterpret_cast<const __nv_bfloat16*>(ws + lay.off_x16),
+                              reinterpret_cast<const __nv_bfloat16*>(dZ), dwf, wst);
       if (rc) return rc;
       LCN_CHECK_CUDA(cudaMemcpyAsync(graw + L.w_off, dwf, sizeof(float) * L.Kin * P, cudaMemcpyDeviceToDevice, wst));
       break;
@@ -2033,66 +2032,51 @@ static int backward_impl(const lcn_model* m, const float* params, char* ws, cons
       break;
     }
     const T* Ain = reinterpret_cast<const T*>(a_buf(ws, lay, l - 1));
-    // gradient w.r.t. the layer input goes to the next free buffer; the block-output gradient D(cur)
-    // of a residual block stays alive until the first layer of the block has been processed.
-    bool second_of_block = (L.res_from >= 0) || (!m->d.residual && (l % 2 == 0));
-    int nxt = second_of_block ? (cur + 1) % 3 : (cur + 1) % 3;
-    const T* addend = nullptr;
-    int keep = cur;
-    if (!second_of_block && m->d.residual) {
-      // first layer of the block: D(cur) is the mid gradient, D(prev) the block-output gradient
-      addend = D((cur + 2) % 3);
-    }
-    {
-      int rc = lcn_tc_wgrad(m, lay, reinterpret_cast<const __nv_bfloat16*>(Ain),
-                            reinterpret_cast<const __nv_bfloat16*>(dZ), graw + L.w_off, wst, kX3);
+    rc = lcn_tc_wgrad(m, lay, reinterpret_cast<const __nv_bfloat16*>(Ain), reinterpret_cast<const __nv_bfloat16*>(dZ),
+                      graw + L.w_off, wst, kX3);
+    if (rc) return rc;
+    LCN_CHECK_CUDA(cudaEventRecord(ax->ev_wg[l & 1], wst));
+    wg_pending[l & 1] = true;
+    if (dp_mode == 1 && l >= LCN_DP_STREAM_FROM) {   // dW_l is final on the side stream: average its joint-pair blocks over the ranks
+      LCN_CHECK_CUDA(cudaStreamWaitEvent(ax->xst, ax->ev_wg[l & 1], 0));
+      rc = lcn_dp_exchange_units(m, graw, l * m->nnz, (l + 1) * m->nnz, 0, 0, m->sm_count, ax->xst);
       if (rc) return rc;
-      if (ax) {
-        LCN_CHECK_CUDA(cudaEventRecord(ax->ev_wg[l & 1], wst));
-        wg_pending[l & 1] = true;
-      }
-      if (dp_stream && l >= LCN_DP_STREAM_FROM) {   // dW_l is final on the side stream: average its joint-pair blocks over the ranks
-        LCN_CHECK_CUDA(cudaStreamWaitEvent(ax->xst, ax->ev_wg[l & 1], 0));
-        rc = lcn_dp_exchange_units(m, graw, l * m->nnz, (l + 1) * m->nnz, 0, 0, m->sm_count, ax->xst);
-        if (rc) return rc;
-        dp_forked = true;
-      }
-      const size_t wofs = (size_t)(l - 1) * m->nnz * FC * FC * 4096 * 2;
-      rc = lcn_tc_gemm(m, lay, l - 1, 1, reinterpret_cast<const __nv_bfloat16*>(dZ), ws + lay.off_wp16b + wofs, nullptr,
-                       reinterpret_cast<const __nv_bfloat16*>(addend), reinterpret_cast<__nv_bfloat16*>(D(nxt)),
-                       nullptr, st, nullptr, nullptr, kX3 ? ws + lay.off_wp16b_lo + wofs : nullptr);
-      if (rc) return rc;
+      dp_forked = true;
     }
+    // the gradient w.r.t. the layer input goes to the next of the three buffers.  The first layer of a residual block
+    // (the one without res_from) adds the block-output gradient, which the block's second layer left in D(cur + 2).
+    const T* addend = m->d.residual && L.res_from < 0 ? D((cur + 2) % 3) : nullptr;
+    const MidWeights w = mid_weights(m, ws, lay, l, 1);
+    rc = lcn_tc_gemm(m, lay, l - 1, 1, reinterpret_cast<const __nv_bfloat16*>(dZ), w.hi, nullptr,
+                     reinterpret_cast<const __nv_bfloat16*>(addend), reinterpret_cast<__nv_bfloat16*>(D((cur + 1) % 3)),
+                     nullptr, st, nullptr, nullptr, w.lo);
+    if (rc) return rc;
     LCN_CHECK_LAUNCH();
-    (void)keep;
-    cur = nxt;
+    cur = (cur + 1) % 3;
   }
   {
     LinTable lb;
     lb.n = m->n_bn;
     for (int l = 0; l < m->n_bn; ++l) lb.w_off[l] = m->L[l].b_off;
     lcn_launch(k_db_reduce, dim3(dim3((P + 63) / 64, m->n_bn)), dim3(256), 0, st, reinterpret_cast<const float*>(ws + lay.off_dbpart),
-                                                              (int)eg, P, graw, lb);
+                                                              ew.grid, P, graw, lb);
     LCN_CHECK_LAUNCH();
   }
-  if (ax) {                          // join: the caller's stream continues after the last weight gradient
-    LCN_CHECK_CUDA(cudaEventRecord(ax->ev_done, wst));
-    LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_done, 0));
-  }
+  // join: the caller's stream continues after the last weight gradient
+  LCN_CHECK_CUDA(cudaEventRecord(ax->ev_done, wst));
+  LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_done, 0));
   if (dp_mode) {
     // the bucket is complete on this stream -> two-shot all-reduce over NVLink peer memory of whatever has not been
     // exchanged yet; after the wait (in stream order) the bucket holds the mean over the ranks
     if (dp_forked) {
       LCN_CHECK_CUDA(cudaEventRecord(ax->ev_xdone, ax->xst));
       LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_xdone, 0));
-      int rc2 = lcn_dp_exchange_units(m, graw, 0, -1, LCN_DP_STREAM_FROM * m->nnz, (m->n_lin - 1) * m->nnz, 0, st);   // all but the streamed layers
-      if (rc2) return rc2;
+      rc = lcn_dp_exchange_units(m, graw, 0, -1, LCN_DP_STREAM_FROM * m->nnz, (m->n_lin - 1) * m->nnz, 0, st);   // all but the streamed layers
     } else {
-      int rc2 = lcn_dp_exchange_units(m, graw, 0, -1, 0, 0, 0, st);
-      if (rc2) return rc2;
+      rc = lcn_dp_exchange_units(m, graw, 0, -1, 0, 0, 0, st);
     }
-    int rc2 = lcn_dp_wait(m, st);
-    if (rc2) return rc2;
+    if (rc) return rc;
+    return lcn_dp_wait(m, st);
   }
   return LCN_OK;
 }
@@ -2108,17 +2092,13 @@ int lcn_launch_backward(const lcn_model* m, const float* params, char* ws, const
 template <typename T>
 static int layer_gemm_impl(const lcn_model* m, const float* params, char* ws, const WsLayout& lay, int l,
                            int transposed, cudaStream_t st) {
-  const int FC = m->FC;
-  constexpr bool kX3 = PathTraits<T>::x3;
   float* part = reinterpret_cast<float*>(ws + lay.off_part);
   const T* Ain = reinterpret_cast<const T*>(transposed ? ws + lay.off_dz : a_buf(ws, lay, l - 1));
   T* Y = reinterpret_cast<T*>(transposed ? ws + lay.off_d + 2 * lay.d_stride : z_buf(ws, lay, l));
-  const size_t wofs = (size_t)(l - 1) * m->nnz * FC * FC * 4096 * 2;
-  const char* wp = ws + (transposed ? lay.off_wp16b : lay.off_wp16f) + wofs;
-  const char* wl = kX3 ? ws + (transposed ? lay.off_wp16b_lo : lay.off_wp16f_lo) + wofs : nullptr;
-  return lcn_tc_gemm(m, lay, l - 1, transposed, reinterpret_cast<const __nv_bfloat16*>(Ain), wp,
+  const MidWeights w = mid_weights(m, ws, lay, l, transposed);
+  return lcn_tc_gemm(m, lay, l - 1, transposed, reinterpret_cast<const __nv_bfloat16*>(Ain), w.hi,
                      transposed ? nullptr : params + m->L[l].b_off, nullptr, reinterpret_cast<__nv_bfloat16*>(Y),
-                     transposed ? nullptr : part, st, nullptr, nullptr, wl);
+                     transposed ? nullptr : part, st, nullptr, nullptr, w.lo);
 }
 int lcn_launch_layer_gemm(const lcn_model* m, const float* params, char* ws, const WsLayout& lay, int layer,
                           int transposed, cudaStream_t st) {
