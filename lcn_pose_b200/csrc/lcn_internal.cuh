@@ -248,11 +248,46 @@ static inline void lcn_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
     }                            \
   } while (0)
 
-// ---- data-parallel exchange (lcn_dp.cu) ----
-int lcn_dp_mode(const lcn_model* m);      // 0: no exchange; 1: streamed behind the weight-gradient GEMMs; 2: one exchange at the end
-int lcn_dp_exchange_units(const lcn_model* m, float* graw, int u0, int u1, int s0, int s1, int max_ctas, cudaStream_t st);
-int lcn_dp_wait(const lcn_model* m, cudaStream_t st);
+// Per-layer weight geometry and the support's pair list, passed to kernels by value
+struct LinTable {
+  int n;
+  int64_t w_off[LCN_MAX_LIN];
+  int32_t Fi[LCN_MAX_LIN], Fo[LCN_MAX_LIN];
+};
+struct PairTable {
+  uint8_t pi[LCN_J * LCN_J], pj[LCN_J * LCN_J];
+};
+static inline LinTable make_lin(const lcn_model* m) {
+  LinTable t;
+  t.n = m->n_lin;
+  for (int l = 0; l < m->n_lin; ++l) {
+    t.w_off[l] = m->L[l].w_off;
+    t.Fi[l] = m->L[l].Fi;
+    t.Fo[l] = m->L[l].Fo;
+  }
+  return t;
+}
+static inline PairTable make_pairs(const lcn_model* m) {
+  PairTable t;
+  for (int i = 0; i < LCN_J; ++i)
+    for (int j = 0; j < LCN_J; ++j)
+      if (m->sup.pair[i][j] >= 0) {
+        t.pi[m->sup.pair[i][j]] = (uint8_t)i;
+        t.pj[m->sup.pair[i][j]] = (uint8_t)j;
+      }
+  return t;
+}
+
+// ---- data-parallel training (lcn_dp.cu) ----
+// Gradient exchange of the backward pass; both are no-ops when the model has no exchange.  After the weight-gradient
+// GEMM of mid layer l has been enqueued on ax->st and ev_wg[l & 1] recorded:
+int lcn_dp_exchange_layer(const lcn_model* m, const float* graw, int l, LcnAux* ax);
+// At the end of the backward pass, once the bucket is complete on `st`: the rest of the exchange, then `st` waits until
+// this rank's bucket holds the mean over the ranks.
+int lcn_dp_exchange_rest(const lcn_model* m, const float* graw, LcnAux* ax, cudaStream_t st);
 void lcn_dp_destroy(lcn_model* m);
+int64_t lcn_grad_compact_count(const lcn_model* m);
+int lcn_launch_grad_compact(const lcn_model* m, float* graw, float* compact, bool unpack, cudaStream_t st);
 // synchronised BatchNorm (lcn_dp_sync_batch_norm): the source of a sync point's local moments
 #define LCN_BN_SYNC_GACC 0      // forward, double[LCN_GACC_REP][F][2] (sum x, sum x^2) of the tensor-core GEMM
 #define LCN_BN_SYNC_MOMENTS 1   // forward, double[F][3] (n, mean, M2) of k_bn_finalize
@@ -286,12 +321,6 @@ int lcn_launch_grad_finalize(const lcn_model* m, const float* params, char* ws, 
 int lcn_launch_adam(const lcn_model* m, float* params, float* mm, float* vv, char* ws, const WsLayout& lay,
                     const float* grads_raw, float lr_t, float b1, float b2, float eps, float reg,
                     const lcn_step_scalars* dyn, cudaStream_t st);
-int64_t lcn_grad_compact_count(const lcn_model* m);
-int lcn_launch_grad_compact(const lcn_model* m, float* graw, float* compact, bool unpack, cudaStream_t st);
-int lcn_launch_dp_exchange(const lcn_model* m, float* const* buckets, float* const* stage_at, float* const* stage_local,
-                           unsigned long long* pushed_local, unsigned long long* const* pushed_at,
-                           unsigned long long* const* done_at, unsigned long long* epoch, unsigned int* ticket, int rank,
-                           int world, int u0, int u1, int s0, int s1, int max_ctas, cudaStream_t st);
 int lcn_launch_layer_gemm(const lcn_model* m, const float* params, char* ws, const WsLayout& lay, int layer,
                           int transposed, cudaStream_t st);
 int lcn_launch_read_tensor(const lcn_model* m, char* ws, const WsLayout& lay, int kind, int layer,

@@ -1,8 +1,8 @@
 // CUDA-core kernels of the LCN hot path: weight preparation (clip_by_norm + mask + pack), the edge
 // layers (17*in_F -> 17*F and 17*F -> 51), BatchNorm statistics / apply, the elementwise half of the backward
-// pass, the fused masked TF1-Adam step, the pack / exchange kernels of data-parallel training, and the
-// orchestration of the forward / backward passes of both arithmetic paths.
-// The tensor-core (tcgen05) mid-layer GEMMs of both paths live in lcn_gemm_tc.cu.
+// pass, the fused masked TF1-Adam step, and the orchestration of the forward / backward passes of both arithmetic
+// paths.  The tensor-core (tcgen05) mid-layer GEMMs of both paths live in lcn_gemm_tc.cu, the data-parallel exchange
+// and the gradient pack / unpack in lcn_dp.cu.
 //
 // Reference semantics implemented here (paths relative to the reference root):
 //   network/models_att.py:534-586 (mask, mask_weights), :588-612 (BN), :630-775 (layers, head),
@@ -25,38 +25,9 @@ struct PathTraits {
   static constexpr bool x3 = std::is_same<T, lcn_sp16>::value;
 };
 
-struct LinTable {
-  int n;
-  int64_t w_off[LCN_MAX_LIN];
-  int32_t Fi[LCN_MAX_LIN], Fo[LCN_MAX_LIN];
-};
-struct PairTable {
-  uint8_t pi[LCN_J * LCN_J], pj[LCN_J * LCN_J];
-};
 struct ConstMask {
   float v[LCN_J * LCN_J];
 };
-
-static LinTable make_lin(const lcn_model* m) {
-  LinTable t;
-  t.n = m->n_lin;
-  for (int l = 0; l < m->n_lin; ++l) {
-    t.w_off[l] = m->L[l].w_off;
-    t.Fi[l] = m->L[l].Fi;
-    t.Fo[l] = m->L[l].Fo;
-  }
-  return t;
-}
-static PairTable make_pairs(const lcn_model* m) {
-  PairTable t;
-  for (int i = 0; i < LCN_J; ++i)
-    for (int j = 0; j < LCN_J; ++j)
-      if (m->sup.pair[i][j] >= 0) {
-        t.pi[m->sup.pair[i][j]] = (uint8_t)i;
-        t.pj[m->sup.pair[i][j]] = (uint8_t)j;
-      }
-  return t;
-}
 
 __device__ __forceinline__ double block_reduce_sum_d(double v, double* sh /* >= 32 */) {
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -1470,259 +1441,6 @@ __global__ void __launch_bounds__(256) k_adam(float* __restrict__ params, float*
   }
 }
 
-// ------------------------------------------------------------------------------------------------
-// packed gradient exchange (include/lcn_b200.h: lcn_model_pack_grads / lcn_model_unpack_grads)
-// blocks [0, nnz * n_lin): one Fi x Fo block of one weight matrix; the remaining blocks: one non-weight tensor each
-// ------------------------------------------------------------------------------------------------
-struct CompactTable {
-  int64_t w_coff[LCN_MAX_LIN];          // compact offset of layer l's first block
-  int n_other;
-  int64_t o_off[LCN_MAX_TENSORS], o_size[LCN_MAX_TENSORS], o_coff[LCN_MAX_TENSORS];
-  int64_t total;
-};
-static CompactTable make_compact(const lcn_model* m) {
-  CompactTable c;
-  memset(&c, 0, sizeof(c));
-  int64_t off = 0;
-  for (int l = 0; l < m->n_lin; ++l) {
-    c.w_coff[l] = off;
-    off += (int64_t)m->nnz * m->L[l].Fi * m->L[l].Fo;
-  }
-  for (int s = 0; s < m->segs.n; ++s) {
-    if (m->segs.s[s].kind == SEG_W) continue;
-    c.o_off[c.n_other] = m->segs.s[s].off;
-    c.o_size[c.n_other] = m->segs.s[s].size;
-    c.o_coff[c.n_other] = off;
-    off += m->segs.s[s].size;
-    ++c.n_other;
-  }
-  c.total = off;
-  return c;
-}
-template <bool UNPACK>
-__global__ void __launch_bounds__(256) k_grad_compact(float* __restrict__ graw, float* __restrict__ compact, LinTable lt,
-                                                      PairTable pt, CompactTable ct, int nnz, int n_lin) {
-  lcn_pdl_prologue();
-  const int b = blockIdx.x;
-  if (b < nnz * n_lin) {
-    const int l = b / nnz, p = b - l * nnz;
-    const int Fi = lt.Fi[l], Fo = lt.Fo[l], Kout = LCN_J * Fo;
-    const int i = pt.pi[p], j = pt.pj[p];
-    float* g = graw + lt.w_off[l];
-    float* c = compact + ct.w_coff[l] + (int64_t)p * Fi * Fo;
-    if ((Fo & 3) == 0) {                  // 16-byte copies: a block row is Fo contiguous floats in both layouts
-      const int q = Fo >> 2;
-      for (int e = threadIdx.x; e < Fi * q; e += 256) {
-        const int fi = e / q, c4 = (e - fi * q) * 4;
-        float4* gp = reinterpret_cast<float4*>(g + (size_t)(i * Fi + fi) * Kout + j * Fo + c4);
-        float4* cp = reinterpret_cast<float4*>(c + fi * Fo + c4);
-        if (UNPACK) *gp = *cp; else *cp = *gp;
-      }
-    } else {
-      for (int e = threadIdx.x; e < Fi * Fo; e += 256) {
-        const int fi = e / Fo, fo = e - fi * Fo;
-        const size_t o = (size_t)(i * Fi + fi) * Kout + j * Fo + fo;
-        if (UNPACK) g[o] = c[e]; else c[e] = g[o];
-      }
-    }
-  } else {
-    const int k = b - nnz * n_lin;
-    float* g = graw + ct.o_off[k];
-    float* c = compact + ct.o_coff[k];
-    for (int64_t e = threadIdx.x; e < ct.o_size[k]; e += 256) {
-      if (UNPACK) g[e] = c[e]; else c[e] = g[e];
-    }
-  }
-}
-
-int64_t lcn_grad_compact_count(const lcn_model* m) { return make_compact(m).total; }
-int lcn_launch_grad_compact(const lcn_model* m, float* graw, float* compact, bool unpack, cudaStream_t st) {
-  const CompactTable ct = make_compact(m);
-  const dim3 grid(m->nnz * m->n_lin + ct.n_other);
-  if (unpack) lcn_launch(k_grad_compact<true>, grid, dim3(256), 0, st, graw, compact, make_lin(m), make_pairs(m), ct, m->nnz, m->n_lin);
-  else lcn_launch(k_grad_compact<false>, grid, dim3(256), 0, st, graw, compact, make_lin(m), make_pairs(m), ct, m->nnz, m->n_lin);
-  LCN_CHECK_LAUNCH();
-  return LCN_OK;
-}
-
-// ------------------------------------------------------------------------------------------------
-// data-parallel exchange (lcn_dp.cu): two-shot all-reduce of the gradient bucket over NVLink peer memory with STORES only.
-// The unit of work is the unit of k_grad_compact -- one Fi x Fo joint-pair block of one weight matrix inside the mask
-// support, or one small tensor -- so the masked-out 40 % of the bucket is never read, never sent.  Units are dealt
-// round-robin to the ranks (owner = unit % world).
-//   k_dp_push    every rank copies its local copy of the units it does NOT own into the owner's staging area (slot
-//                [sender], packed at the unit's k_grad_compact offset): 16-byte peer stores, posted, no round trip;
-//                the last CTA publishes pushed[me] = epoch at every peer
-//   k_dp_reduce  the owner waits for pushed[p] >= epoch from every peer, then for each of its units adds its own block and
-//                the world-1 staged copies (all LOCAL reads) in a fixed order -- every rank ends up with bit-identical
-//                gradients -- and stores the mean into ALL `world` parameter-layout buckets (peer stores again); the
-//                last CTA publishes done[me] = epoch at every peer
-// The pull variant (reduce-scatter by peer LOADS straight out of the peers' buckets, no staging slots) was built and
-// measured first: 0.632 ms per step at 2 GPUs and 0.682 ms at 8, against 0.631 / 0.676 ms for this one -- the same within
-// run-to-run noise; both move 2 (world-1)/world of the bucket per GPU at ~340 GB/s of NVLink egress.  Stores are kept
-// because they are posted writes whose completion does not depend on a round trip through a busy peer.
-// Unit sets of different ranks are disjoint, so writing the mean in place into every bucket is race free: a rank reads a
-// peer-owned unit of its own bucket only in k_dp_push, and the owner overwrites it only after pushed[] from everybody.
-// ------------------------------------------------------------------------------------------------
-struct DpArgs {
-  float* g[8];                            // the `world` parameter-layout gradient buckets (g[rank] is local)
-  float* stage[8];                        // push: stage[q] = rank q's staging slot for THIS rank; reduce: local slot of sender p
-  unsigned long long* wait_local;         // [8] local flags to wait for (reduce: pushed[]; unused in push)
-  unsigned long long* signal_at[8];       // the flag this kernel publishes at every rank (push: pushed[me]; reduce: done[me])
-  unsigned long long* epoch;              // local epoch counter (push increments it)
-  unsigned int* ticket;                   // local CTA counter
-  int rank, world;
-};
-// End of an exchange kernel: every block has fenced its (peer) stores and takes a ticket; the last block publishes the
-// epoch at every rank, one thread per rank -- the release stores travel over NVLink concurrently instead of one round
-// trip after the other (8 ranks: one store latency instead of eight on the exposed end of the step).
-__device__ __forceinline__ void dp_finish(const DpArgs& d, unsigned long long e, bool bump_epoch) {
-  __shared__ int s_last;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const bool last = atomicAdd(d.ticket, 1u) == gridDim.x - 1;
-    if (last) {
-      *d.ticket = 0u;
-      if (bump_epoch) *d.epoch = e;
-      __threadfence_system();
-    }
-    s_last = last ? 1 : 0;
-  }
-  __syncthreads();
-  if (s_last && (int)threadIdx.x < d.world)
-    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(d.signal_at[threadIdx.x]), "l"(e) : "memory");
-}
-// geometry of unit b: dense offset of its first element, rows x cols, dense row pitch, offset in the packed order
-struct DpUnit {
-  size_t dense, packed;
-  int rows, cols, pitch;
-};
-__device__ __forceinline__ DpUnit dp_unit(int b, const LinTable& lt, const PairTable& pt, const CompactTable& ct, int nnz, int n_lin) {
-  DpUnit u;
-  if (b < nnz * n_lin) {
-    const int l = b / nnz, p = b - l * nnz;
-    const int Fi = lt.Fi[l], Fo = lt.Fo[l];
-    u.rows = Fi; u.cols = Fo; u.pitch = LCN_J * Fo;
-    u.dense = lt.w_off[l] + (size_t)(pt.pi[p] * Fi) * u.pitch + pt.pj[p] * Fo;
-    u.packed = ct.w_coff[l] + (size_t)p * Fi * Fo;
-  } else {
-    const int k = b - nnz * n_lin;
-    u.rows = 1; u.cols = (int)ct.o_size[k]; u.pitch = u.cols;
-    u.dense = ct.o_off[k];
-    u.packed = ct.o_coff[k];
-  }
-  return u;
-}
-// Both kernels work on the unit range [u0, u1) minus [s0, s1): the whole bucket, the units of one weight matrix when the
-// exchange is streamed behind the weight-gradient GEMMs (lcn_dp.cu), or what is left after those.
-__global__ void __launch_bounds__(256) k_dp_push(DpArgs d, LinTable lt, PairTable pt, CompactTable ct, int nnz, int n_lin,
-                                                 int u0, int u1, int s0, int s1) {
-  lcn_pdl_prologue();
-  const unsigned long long e = *d.epoch + 1;          // (every block reads the old value: the last block stores the new one)
-  const float* mine = d.g[d.rank];
-  for (int b = u0 + blockIdx.x; b < u1; b += gridDim.x) {
-    const int owner = b % d.world;
-    if (owner == d.rank || (b >= s0 && b < s1)) continue;
-    const DpUnit u = dp_unit(b, lt, pt, ct, nnz, n_lin);
-    float* dst = d.stage[owner] + u.packed;
-    if ((u.cols & 3) == 0 && (u.dense & 3) == 0 && (u.packed & 3) == 0) {
-      const int q = u.cols >> 2;
-      for (int t = threadIdx.x; t < u.rows * q; t += 256) {
-        const int r = t / q, c4 = (t - r * q) * 4;
-        *reinterpret_cast<float4*>(dst + r * u.cols + c4) = *reinterpret_cast<const float4*>(mine + u.dense + (size_t)r * u.pitch + c4);
-      }
-    } else {
-      for (int t = threadIdx.x; t < u.rows * u.cols; t += 256) {
-        const int r = t / u.cols, c = t - r * u.cols;
-        dst[t] = mine[u.dense + (size_t)r * u.pitch + c];
-      }
-    }
-  }
-  dp_finish(d, e, /*bump_epoch=*/true);
-}
-template <int W>
-__global__ void __launch_bounds__(256) k_dp_reduce(DpArgs d, LinTable lt, PairTable pt, CompactTable ct, int nnz, int n_lin,
-                                                   int u0, int u1, int s0, int s1) {
-  lcn_pdl_prologue();
-  const unsigned long long e = *d.epoch;
-  if ((int)threadIdx.x < W && (int)threadIdx.x != d.rank) {
-    unsigned long long v, spins = 0;
-    do {
-      asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(d.wait_local + threadIdx.x) : "memory");
-      if (v < e && ++spins > (1ull << 28)) { printf("lcn_dp: wait for a peer's pushed flag timed out\n"); __trap(); }
-    } while (v < e);
-  }
-  __syncthreads();
-  const float inv = 1.f / (float)W;
-  float* mine = d.g[d.rank];
-  const int first = u0 + ((d.rank - u0 % W) + W) % W;          // first unit >= u0 this rank owns (owner = unit % W)
-  for (int b = first + blockIdx.x * W; b < u1; b += gridDim.x * W) {
-    if (b >= s0 && b < s1) continue;
-    const DpUnit u = dp_unit(b, lt, pt, ct, nnz, n_lin);
-    if ((u.cols & 3) == 0 && (u.dense & 3) == 0 && (u.packed & 3) == 0) {
-      const int q = u.cols >> 2;
-      for (int t = threadIdx.x; t < u.rows * q; t += 256) {
-        const int r = t / q, c4 = (t - r * q) * 4;
-        const size_t off = u.dense + (size_t)r * u.pitch + c4;
-        float4 v[W];
-#pragma unroll
-        for (int p = 0; p < W; ++p)                    // rank order, the same on every rank: bit-identical means
-          v[p] = p == d.rank ? *reinterpret_cast<const float4*>(mine + off)
-                             : __ldcg(reinterpret_cast<const float4*>(d.stage[p] + u.packed + r * u.cols + c4));
-        float4 a = v[0];
-#pragma unroll
-        for (int p = 1; p < W; ++p) { a.x += v[p].x; a.y += v[p].y; a.z += v[p].z; a.w += v[p].w; }
-        a.x *= inv; a.y *= inv; a.z *= inv; a.w *= inv;
-#pragma unroll
-        for (int p = 0; p < W; ++p) *reinterpret_cast<float4*>(d.g[p] + off) = a;
-      }
-    } else {
-      for (int t = threadIdx.x; t < u.rows * u.cols; t += 256) {
-        const int r = t / u.cols, c = t - r * u.cols;
-        const size_t off = u.dense + (size_t)r * u.pitch + c;
-        float a = 0.f;
-        for (int p = 0; p < W; ++p) a += p == d.rank ? mine[off] : __ldcg(d.stage[p] + u.packed + t);
-        a *= inv;
-        for (int p = 0; p < W; ++p) d.g[p][off] = a;
-      }
-    }
-  }
-  dp_finish(d, e, /*bump_epoch=*/false);
-}
-// buckets[p], stage_at[q] (rank q's slot for this rank), stage_local[p] (this rank's slot for sender p)
-int lcn_launch_dp_exchange(const lcn_model* m, float* const* buckets, float* const* stage_at, float* const* stage_local,
-                           unsigned long long* pushed_local, unsigned long long* const* pushed_at,
-                           unsigned long long* const* done_at, unsigned long long* epoch, unsigned int* ticket, int rank,
-                           int world, int u0, int u1, int s0, int s1, int max_ctas, cudaStream_t st) {
-  const CompactTable ct = make_compact(m);
-  DpArgs a, r;
-  memset(&a, 0, sizeof(a));
-  for (int p = 0; p < world; ++p) { a.g[p] = buckets[p]; a.stage[p] = stage_at[p]; a.signal_at[p] = pushed_at[p]; }
-  a.epoch = epoch;
-  a.ticket = ticket;
-  a.rank = rank;
-  a.world = world;
-  r = a;
-  for (int p = 0; p < world; ++p) { r.stage[p] = stage_local[p]; r.signal_at[p] = done_at[p]; }
-  r.wait_local = pushed_local;
-  const int n_all = m->nnz * m->n_lin + ct.n_other;
-  if (u1 < 0 || u1 > n_all) u1 = n_all;
-  const int n_units = u1 - u0 - std::max(0, std::min(s1, u1) - std::max(s0, u0));
-  if (max_ctas <= 0) max_ctas = 4 * m->sm_count;
-  const dim3 gpush(std::max(1, std::min(n_units, max_ctas)));
-  const dim3 gred(std::max(1, std::min((n_units + world - 1) / world, max_ctas)));
-  lcn_launch(k_dp_push, gpush, dim3(256), 0, st, a, make_lin(m), make_pairs(m), ct, m->nnz, m->n_lin, u0, u1, s0, s1);
-  switch (world) {
-    case 2: lcn_launch(k_dp_reduce<2>, gred, dim3(256), 0, st, r, make_lin(m), make_pairs(m), ct, m->nnz, m->n_lin, u0, u1, s0, s1); break;
-    case 4: lcn_launch(k_dp_reduce<4>, gred, dim3(256), 0, st, r, make_lin(m), make_pairs(m), ct, m->nnz, m->n_lin, u0, u1, s0, s1); break;
-    case 8: lcn_launch(k_dp_reduce<8>, gred, dim3(256), 0, st, r, make_lin(m), make_pairs(m), ct, m->nnz, m->n_lin, u0, u1, s0, s1); break;
-    default: lcn_set_error("data-parallel exchange: world size %d not in {2, 4, 8}", world); return LCN_EINVAL;
-  }
-  LCN_CHECK_LAUNCH();
-  return LCN_OK;
-}
-
 static int launch_grad_chain(const lcn_model* m, const float* params, char* ws, const WsLayout& lay,
                              const float* graw, cudaStream_t st, int zero_norm2) {
   LayerScalars* sc = reinterpret_cast<LayerScalars*>(ws + lay.off_scalars);
@@ -1910,12 +1628,6 @@ int lcn_launch_forward(const FwdArgs& a) {
   return a.m->d.path == LCN_PATH_BF16 ? forward_impl<__nv_bfloat16>(a) : forward_impl<lcn_sp16>(a);
 }
 
-// Streamed data-parallel exchange, measured at 2 GPUs (profiles/r2/dp_streamed_variants.txt): layers >= LCN_DP_STREAM_FROM
-// are exchanged behind their weight-gradient GEMM with one CTA per SM -- 8 CTAs: 0.973 ms/step, 24: 0.656, 64: 0.623,
-// >= 128: 0.618 (the exchange has to keep up with one weight gradient every ~43 us; its CTAs are short-lived and do not
-// slow the backward pass measurably); layer 1, whose gradient is the last to finish, goes with the first / last layer and
-// the small tensors in one full-width exchange at the end (streaming it as well: 0.621).
-#define LCN_DP_STREAM_FROM 2
 template <typename T>
 static int backward_impl(const lcn_model* m, const float* params, char* ws, const WsLayout& lay, const float* x,
                          const float* labels, float rate, uint64_t seed, uint64_t step, float* loss,
@@ -1928,12 +1640,7 @@ static int backward_impl(const lcn_model* m, const float* params, char* ws, cons
   int rc = lcn_aux_get(m, &ax);
   if (rc) return rc;
   cudaStream_t wst = ax->st;
-  // data parallel (lcn_dp.cu): in mode 1 the mean of every mid-layer weight gradient is exchanged over NVLink on a third
-  // stream as soon as its GEMM has finished, under the rest of the backward pass; what is left for the end is the
-  // first and last layer and the small tensors (< 2 % of the bucket)
-  const int dp_mode = lcn_dp_mode(m);
   const bool bn_sync = lcn_bn_sync_on(m);
-  bool dp_forked = false;
   bool wg_pending[2] = {false, false};
   const int64_t blast = m->L[m->n_lin - 1].b_off;     // last-layer bias gradient: accumulated by k_loss_dout (caller's stream)
   // fork at the very start: the 4 B/parameter clear of the gradient bucket (the weight-gradient GEMMs reduce-add
@@ -2037,12 +1744,8 @@ static int backward_impl(const lcn_model* m, const float* params, char* ws, cons
     if (rc) return rc;
     LCN_CHECK_CUDA(cudaEventRecord(ax->ev_wg[l & 1], wst));
     wg_pending[l & 1] = true;
-    if (dp_mode == 1 && l >= LCN_DP_STREAM_FROM) {   // dW_l is final on the side stream: average its joint-pair blocks over the ranks
-      LCN_CHECK_CUDA(cudaStreamWaitEvent(ax->xst, ax->ev_wg[l & 1], 0));
-      rc = lcn_dp_exchange_units(m, graw, l * m->nnz, (l + 1) * m->nnz, 0, 0, m->sm_count, ax->xst);
-      if (rc) return rc;
-      dp_forked = true;
-    }
+    rc = lcn_dp_exchange_layer(m, graw, l, ax);   // data parallel: dW_l is final on the side stream
+    if (rc) return rc;
     // the gradient w.r.t. the layer input goes to the next of the three buffers.  The first layer of a residual block
     // (the one without res_from) adds the block-output gradient, which the block's second layer left in D(cur + 2).
     const T* addend = m->d.residual && L.res_from < 0 ? D((cur + 2) % 3) : nullptr;
@@ -2065,20 +1768,7 @@ static int backward_impl(const lcn_model* m, const float* params, char* ws, cons
   // join: the caller's stream continues after the last weight gradient
   LCN_CHECK_CUDA(cudaEventRecord(ax->ev_done, wst));
   LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_done, 0));
-  if (dp_mode) {
-    // the bucket is complete on this stream -> two-shot all-reduce over NVLink peer memory of whatever has not been
-    // exchanged yet; after the wait (in stream order) the bucket holds the mean over the ranks
-    if (dp_forked) {
-      LCN_CHECK_CUDA(cudaEventRecord(ax->ev_xdone, ax->xst));
-      LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_xdone, 0));
-      rc = lcn_dp_exchange_units(m, graw, 0, -1, LCN_DP_STREAM_FROM * m->nnz, (m->n_lin - 1) * m->nnz, 0, st);   // all but the streamed layers
-    } else {
-      rc = lcn_dp_exchange_units(m, graw, 0, -1, 0, 0, 0, st);
-    }
-    if (rc) return rc;
-    return lcn_dp_wait(m, st);
-  }
-  return LCN_OK;
+  return lcn_dp_exchange_rest(m, graw, ax, st);   // data parallel: the bucket holds the mean over the ranks after this
 }
 
 int lcn_launch_backward(const lcn_model* m, const float* params, char* ws, const WsLayout& lay, const float* x,

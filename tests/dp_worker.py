@@ -4,7 +4,9 @@ on `world` GPUs, checked on hardware --
     compared against an fp64 mean of the all-gathered local buckets),
   * after K graph-replayed DP steps every replica holds bit-identical parameters and Adam moments,
   * the replicas' trajectory equals a single process that averages the same per-rank gradients itself.
-Prints one JSON line per rank; exit code 0 = all assertions held."""
+argv: mode (p2p | p2p-end | packed).  LCN_DP_SHARE_GPU=1: every rank on device 0 (one-GPU machines: the exchange then
+goes through CUDA IPC within one device, the rendezvous through gloo).  Prints one JSON line per rank; exit code 0 = all
+assertions held."""
 import json
 import os
 import sys
@@ -31,9 +33,15 @@ def main():
         import faulthandler
         faulthandler.dump_traceback_later(float(os.environ["LCN_HANG_TRACE"]), exit=False)
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
+    shared = os.environ.get("LCN_DP_SHARE_GPU") == "1"
+    if shared:
+        local = 0
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
-    dist.init_process_group("nccl", device_id=dev)
+    if shared:
+        dist.init_process_group("gloo")
+    else:
+        dist.init_process_group("nccl", device_id=dev)
     nm = params_help.get_neighbour_matrix_by_hand(params_help.filter_hub.neighbour_dict_set[0], knn=3)
     mode = sys.argv[1] if len(sys.argv) > 1 else "packed"
     steps, n = 5, 512
