@@ -271,10 +271,10 @@ WsLayout lcn_ws_layout(const lcn_model* m, int64_t n_rows, int bn_group, int tra
   w.off_wm_last = take(sizeof(float) * m->L[m->n_lin - 1].Kin * m->L[m->n_lin - 1].Kout);
   size_t n_mid = m->n_lin - 2;
   size_t sub = (size_t)m->nnz * m->FC * m->FC * 4096;
-  w.off_wp32 = take(sizeof(float) * n_mid * sub);
+  const bool x3 = m->d.path == LCN_PATH_FP32;          // fp32 copy for the weight tap, and the lo parts of split bf16
+  w.off_wp32 = take(x3 ? sizeof(float) * n_mid * sub : 0);
   w.off_wp16f = take(2 * n_mid * sub);
   w.off_wp16b = take(2 * n_mid * sub);
-  const bool x3 = m->d.path == LCN_PATH_FP32;          // split-bf16 operands: the lo parts of the packed blocks
   w.off_wp16f_lo = take(x3 ? 2 * n_mid * sub : 0);
   w.off_wp16b_lo = take(x3 ? 2 * n_mid * sub : 0);
   w.off_wl16f = take((size_t)LCN_J * m->FC * 8192);

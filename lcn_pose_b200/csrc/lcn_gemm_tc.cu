@@ -801,7 +801,7 @@ int lcn_tc_gemm(const lcn_model* m, const WsLayout& lay, int mid_index, int tran
 }
 
 // last layer (17*F -> 51) + output head on the tensor cores: one N-side chunk (51 columns padded to 64),
-// every K chunk present; weights packed by k_pack_last16 as one 64x64 block per K chunk.
+// every K chunk present; weights packed by k_pack_edges as one 64x64 block per K chunk.
 int lcn_tc_head(const lcn_model* m, const WsLayout& lay, const __nv_bfloat16* A, const char* wpacked,
                 const float* bias, const float* x, float* out_user, float* out_ws, cudaStream_t st) {
   TcParams p;

@@ -116,7 +116,7 @@ struct WsLayout {
   size_t off_pairdot;                // float[n_lin][289]  <dWm, W> per support pair
   size_t off_loss;                   // double[2]
   size_t off_wm_first, off_wm_last;  // dense masked fp32 effective weights of the edge layers
-  size_t off_wp32;                   // fp32 packed mid-layer blocks  [mid][pair][FC][FC][64][64]
+  size_t off_wp32;                   // fp32 packed mid-layer blocks  [mid][pair][FC][FC][64][64] (fp32-parity path)
   size_t off_wp16f, off_wp16b;       // bf16 UMMA-layout packed blocks (forward / transposed)
   size_t off_wp16f_lo, off_wp16b_lo; // their lo parts (split-bf16 path only)
   size_t off_wl16f, off_wl16b;       // bf16 packed last-layer weights: per K chunk [64 n][64 k] / per N chunk

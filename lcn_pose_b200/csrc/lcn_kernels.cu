@@ -66,8 +66,9 @@ __global__ void k_sumsq(const float* __restrict__ params, LinTable lt, LayerScal
 }
 
 // mask = softmax(var, axis=0) * support (models_att.py:569-571) or the constant; per-layer clip scale.
-// The weight-pack kernels evaluate these two helpers themselves (one thread per block), so that k_mask_scalars is not a
-// launch of its own in front of them on the tail of every train step; it remains for models without mid layers.
+// The weight-pack kernels evaluate these two helpers themselves (one thread per block), so that storing the mask values
+// and scalars is not a launch of its own in front of them on the tail of every train step: block (0, 0, 0) of
+// k_pack_edges stores them (lcn_write_mask_scalars) for the kernels that follow the weight preparation.
 __device__ __forceinline__ float lcn_mask_value(const float* __restrict__ params, int64_t mask_off, const ConstMask& cmask,
                                                 const SupportBits& sup, int i, int j) {
   if (!((sup.row[i] >> j) & 1u)) return 0.f;
@@ -96,38 +97,17 @@ __device__ __forceinline__ void lcn_write_mask_scalars(const float* __restrict__
     sc[t].clipped = clip ? 1.f : 0.f;
   }
 }
-__global__ void k_mask_scalars(const float* __restrict__ params, int64_t mask_off, SupportBits sup,
-                               ConstMask cmask, int n_lin, int max_norm,
-                               LayerScalars* sc, float* mask_out) {
-  lcn_pdl_prologue();
-  lcn_write_mask_scalars(params, mask_off, cmask, sup, n_lin, max_norm, sc, mask_out, (int)threadIdx.x);
-}
-
-// dense masked effective weight of an edge layer: Wm = W * inv_norm * mask[i,j]
-__global__ void k_pack_edge(const float* __restrict__ w, int Fi, int Fo, const LayerScalars* sc, int l,
-                            const float* __restrict__ mask, float* __restrict__ wm) {
-  lcn_pdl_prologue();
-  int Kout = LCN_J * Fo;
-  int64_t n = (int64_t)LCN_J * Fi * Kout;
-  float inv = sc[l].inv_norm;
-  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
-    int r = (int)(e / Kout), c = (int)(e - (int64_t)r * Kout);
-    wm[e] = w[e] * inv * mask[(r / Fi) * LCN_J + c / Fo];
-  }
-}
-
-// packed 64x64 sub-blocks of the mid layers.  grid (nnz*FC*FC, n_mid), 256 threads.
-//   wp32 : [mid][pair][hi][ho][fi][fo] fp32                (CUDA-core GEMMs)
+// packed 64x64 sub-blocks of the mid layers.  grid (nnz*FC*FC, n_mid), 256 threads.  Every block derives its own
+// scale from ||W||^2 and the mask variable (see lcn_mask_value).
+//   wp32 : [mid][pair][hi][ho][fi][fo] fp32, when given (the mid-layer weight tap of the fp32-parity path)
 //   wp16f: bf16, UMMA K-major SWIZZLE_128B image of B[n=fo][k=fi], input-chunk-major order
 //   wp16b: bf16, same for the transposed operand B[n=fi][k=fo], output-chunk-major order
 __global__ void __launch_bounds__(256) k_pack_mid(const float* __restrict__ params, LinTable lt, PairTable pt,
-                                                  SupportBits sup, const LayerScalars* sc,
-                                                  const float* __restrict__ mask, int F, int FC, int nnz,
+                                                  SupportBits sup, const LayerScalars* sc, int F, int FC, int nnz,
                                                   float* __restrict__ wp32, __nv_bfloat16* __restrict__ wp16f,
                                                   __nv_bfloat16* __restrict__ wp16b, __nv_bfloat16* __restrict__ wp16f_lo,
-                                                  __nv_bfloat16* __restrict__ wp16b_lo, int write32, int write16,
-                                                  int64_t mask_off, ConstMask cmask, int n_lin, int max_norm,
-                                                  LayerScalars* sc_out, float* mask_out) {
+                                                  __nv_bfloat16* __restrict__ wp16b_lo, int64_t mask_off, ConstMask cmask,
+                                                  int max_norm) {
   lcn_pdl_prologue();
   __shared__ float tile[64][65];     // tile[fi][fo], scaled
   __shared__ float s_scale;
@@ -136,27 +116,20 @@ __global__ void __launch_bounds__(256) k_pack_mid(const float* __restrict__ para
   int p = sb / (FC * FC), hi = (sb / FC) % FC, ho = sb % FC;
   int i = pt.pi[p], j = pt.pj[p];
   int P = LCN_J * F;
-  // mask_out != nullptr: this launch stands in for k_mask_scalars -- every block derives its own scale from ||W||^2 and
-  // the mask variable, block (0, 0) also stores the 289 mask values and the per-layer scalars for the kernels that follow
   if (threadIdx.x == 0)
-    s_scale = mask_out != nullptr ? lcn_inv_norm(sc, l, max_norm, nullptr) * lcn_mask_value(params, mask_off, cmask, sup, i, j)
-                                  : sc[l].inv_norm * mask[i * LCN_J + j];
+    s_scale = lcn_inv_norm(sc, l, max_norm, nullptr) * lcn_mask_value(params, mask_off, cmask, sup, i, j);
   __syncthreads();
   const float scale = s_scale;
-  if (mask_out != nullptr && blockIdx.x == 0 && blockIdx.y == 0)
-    for (int t = threadIdx.x; t < LCN_J * LCN_J; t += blockDim.x)
-      lcn_write_mask_scalars(params, mask_off, cmask, sup, n_lin, max_norm, sc_out, mask_out, t);
   const float* w = params + lt.w_off[l] + (size_t)(i * F + hi * 64) * P + j * F + ho * 64;
   size_t mid_sb = (size_t)nnz * FC * FC;
-  float* d32 = wp32 + ((size_t)mid * mid_sb + sb) * 4096;
+  float* d32 = wp32 ? wp32 + ((size_t)mid * mid_sb + sb) * 4096 : nullptr;
   for (int f4 = threadIdx.x; f4 < 1024; f4 += 256) {     // coalesced 16-byte loads of the 64x64 block
     int fi = f4 >> 4, c4 = (f4 & 15) * 4;
     float4 v = *reinterpret_cast<const float4*>(w + (size_t)fi * P + c4);
     v.x *= scale; v.y *= scale; v.z *= scale; v.w *= scale;
     tile[fi][c4] = v.x; tile[fi][c4 + 1] = v.y; tile[fi][c4 + 2] = v.z; tile[fi][c4 + 3] = v.w;
-    if (write32) *reinterpret_cast<float4*>(d32 + fi * 64 + c4) = v;
+    if (d32 != nullptr) *reinterpret_cast<float4*>(d32 + fi * 64 + c4) = v;
   }
-  if (!write16) return;
   __syncthreads();
   // destination sub-block slots
   int base_i = 0, base_j = 0;
@@ -196,49 +169,24 @@ __global__ void __launch_bounds__(256) k_pack_mid(const float* __restrict__ para
   }
 }
 
-// bf16 images of the last layer's masked weight for the tensor-core head (one 64x64 block per 64-channel chunk):
-//   wl16f[kc]: B[n = output column (51 padded to 64)][k = channel]   (forward:  out = A * Wm4)
-//   wl16b[kc]: B[n = channel][k = output column]                     (dgrad:    dA = dOut * Wm4^T)
-__global__ void k_pack_last16(const float* __restrict__ wm_last, __nv_bfloat16* __restrict__ wl16f,
-                              __nv_bfloat16* __restrict__ wl16b) {
-  lcn_pdl_prologue();
-  int kc = blockIdx.x;
-  // grid (chunks, 4): a CTA converts 16 channel rows; consecutive threads read consecutive output columns
-  for (int e = blockIdx.y * 1024 + threadIdx.x; e < (int)(blockIdx.y + 1) * 1024; e += blockDim.x) {
-    int k = e >> 6, n = e & 63;      // n: output column jc, k: channel within chunk
-    float v = n < 51 ? wm_last[(size_t)(kc * 64 + k) * 51 + n] : 0.f;
-    __nv_bfloat16 h = __float2bfloat16_rn(v);
-    wl16f[(size_t)kc * 4096 + n * 64 + ((((k >> 3) ^ (n & 7)) << 3) | (k & 7))] = h;
-    wl16b[(size_t)kc * 4096 + k * 64 + ((((n >> 3) ^ (k & 7)) << 3) | (n & 7))] = h;
-  }
-}
-
-// bf16 image of the first layer's masked weight for the fused inference kernel: one 64x64 block per output
-// chunk, B[n = output column of the chunk][k = input feature (17*in_F used, zero padded to 64)]
-__global__ void k_pack_first16(const float* __restrict__ wm_first, int Kin, int P, __nv_bfloat16* __restrict__ wf16) {
-  lcn_pdl_prologue();
-  int oc = blockIdx.x;
-  for (int e = blockIdx.y * 1024 + threadIdx.x; e < (int)(blockIdx.y + 1) * 1024; e += blockDim.x) {
-    int k = e >> 6, n = e & 63;      // consecutive threads read consecutive output columns of input feature k
-    float v = k < Kin ? wm_first[(size_t)k * P + oc * 64 + n] : 0.f;
-    wf16[(size_t)oc * 4096 + n * 64 + ((((k >> 3) ^ (n & 7)) << 3) | (k & 7))] = __float2bfloat16_rn(v);
-  }
-}
-
-// Both edge layers in ONE launch (replaces k_pack_edge x 2 + k_pack_first16 + k_pack_last16 when 17*in_F <= 64): the
-// dense masked weights Wm = W * inv_norm * mask[i,j] in fp32 (CUDA-core first layer / head of the fp32-parity path, parity
-// taps) and, when the bf16 pointers are given, their tensor-core tiles.  grid (17*FC, 4, 2): z = 0 first layer (x = output
-// chunk), z = 1 last layer (x = channel chunk); y = 16 of the 64 rows of the tile.  Scales from ||W||^2 and the mask
-// variable directly (see lcn_mask_value), so the launch does not wait for k_mask_scalars.
+// Both edge layers in one launch (17*in_F <= 64): the dense masked weights Wm = W * inv_norm * mask[i,j] in fp32
+// (CUDA-core first layer / head of the fp32-parity path, parity taps) and, when the bf16 pointers are given, their
+// tensor-core tiles: wf16 one 64x64 block per output chunk of the first layer, B[n = output column][k = input feature,
+// zero padded to 64]; wl16f / wl16b one block per channel chunk of the last layer, B[n = output column (51 padded to 64)]
+// [k = channel] for the forward pass and B[n = channel][k = output column] for dgrad.  grid (17*FC, 4, 2): z = 0 first
+// layer (x = output chunk), z = 1 last layer (x = channel chunk); y = 16 of the 64 rows of the tile.  Scales from ||W||^2
+// and the mask variable directly (see lcn_mask_value); block (0, 0, 0) also stores the 289 mask values and the
+// per-layer scalars.
 __global__ void __launch_bounds__(256) k_pack_edges(const float* __restrict__ params, int64_t w_first, int64_t w_last,
-                                                    int in_F, int F, int P, int last, const LayerScalars* sc,
+                                                    int in_F, int F, int P, int n_lin, LayerScalars* sc,
                                                     int64_t mask_off, ConstMask cmask, SupportBits sup, int max_norm,
+                                                    float* __restrict__ mask_out,
                                                     float* __restrict__ wm_first, float* __restrict__ wm_last,
                                                     __nv_bfloat16* __restrict__ wf16, __nv_bfloat16* __restrict__ wl16f,
                                                     __nv_bfloat16* __restrict__ wl16b) {
   lcn_pdl_prologue();
   __shared__ float s_m[LCN_J];       // mask column / row of this tile, times inv_norm
-  const int x = blockIdx.x;
+  const int x = blockIdx.x, last = n_lin - 1;
   if (blockIdx.z == 0) {
     // first layer: rows k = input feature (joint i = k / in_F), columns of output chunk x (joint j = x*64 / F)
     const int Kin = LCN_J * in_F, j = (x * 64) / F;
@@ -278,6 +226,11 @@ __global__ void __launch_bounds__(256) k_pack_edges(const float* __restrict__ pa
       }
     }
   }
+  // after the tiles and not unrolled: the kernel stays at 32 registers
+  if (x == 0 && blockIdx.y == 0 && blockIdx.z == 0)
+#pragma unroll 1
+    for (int t = threadIdx.x; t < LCN_J * LCN_J; t += blockDim.x)
+      lcn_write_mask_scalars(params, mask_off, cmask, sup, n_lin, max_norm, sc, mask_out, t);
 }
 
 // side stream + events of the model (LcnAux), created on first use under aux.mu (held by the caller).  A creation that
@@ -336,27 +289,8 @@ int lcn_launch_prepare(const lcn_model* m, const float* params, char* ws, const 
   int n_mid = m->n_lin - 2;
   const bool x3 = m->d.path == LCN_PATH_FP32;
   const bool bf = m->d.path == LCN_PATH_BF16;
-  if (n_mid == 0) {
-    // no mid layers: k_mask_scalars, then each edge layer (-> bf16 tiles), in order on the caller's stream
-    lcn_launch(k_mask_scalars, dim3(1), dim3(320), 0, st, params, m->mask_off, m->sup, cmask, m->n_lin, m->d.max_norm, sc, mask);
-    LCN_CHECK_LAUNCH();
-    lcn_launch(k_pack_edge, dim3(64), dim3(256), 0, st, params + m->L[0].w_off, m->L[0].Fi, m->L[0].Fo, sc, 0, mask,
-                                    reinterpret_cast<float*>(ws + lay.off_wm_first));
-    if (bf)
-      lcn_launch(k_pack_first16, dim3(LCN_J * m->FC, 4), dim3(256), 0, st, reinterpret_cast<const float*>(ws + lay.off_wm_first), m->L[0].Kin,
-                                                    m->P, reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wf16));
-    lcn_launch(k_pack_edge, dim3(64), dim3(256), 0, st, params + m->L[last].w_off, m->L[last].Fi, m->L[last].Fo, sc, last, mask,
-                                    reinterpret_cast<float*>(ws + lay.off_wm_last));
-    if (bf)
-      lcn_launch(k_pack_last16, dim3(LCN_J * m->FC, 4), dim3(256), 0, st, reinterpret_cast<const float*>(ws + lay.off_wm_last),
-                                                   reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wl16f),
-                                                   reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wl16b));
-    LCN_CHECK_LAUNCH();
-    return LCN_OK;
-  }
-  // With mid layers the weight preparation is two concurrent launches: k_pack_mid on the caller's stream (it also
-  // stores the mask values and the per-layer scalars for the kernels that follow) and k_pack_edges on the model's side
-  // stream.
+  // The weight preparation is k_pack_edges on the model's side stream (it also stores the mask values and the per-layer
+  // scalars for the kernels that follow) beside k_pack_mid on the caller's stream, for models with mid layers.
   std::lock_guard<std::mutex> aux_lock(m->aux.mu);
   LcnAux* ax;
   int rc = lcn_aux_get(m, &ax);
@@ -364,20 +298,20 @@ int lcn_launch_prepare(const lcn_model* m, const float* params, char* ws, const 
   LCN_CHECK_CUDA(cudaEventRecord(ax->ev_go, st));
   LCN_CHECK_CUDA(cudaStreamWaitEvent(ax->st, ax->ev_go, 0));
   lcn_launch(k_pack_edges, dim3(LCN_J * m->FC, 4, 2), dim3(256), 0, ax->st, params, m->L[0].w_off, m->L[last].w_off, m->d.in_F,
-             m->d.F, m->P, last, static_cast<const LayerScalars*>(sc), m->mask_off, cmask, m->sup, m->d.max_norm,
+             m->d.F, m->P, m->n_lin, sc, m->mask_off, cmask, m->sup, m->d.max_norm, mask,
              reinterpret_cast<float*>(ws + lay.off_wm_first), reinterpret_cast<float*>(ws + lay.off_wm_last),
              bf ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wf16) : nullptr,
              bf ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wl16f) : nullptr,
              bf ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wl16b) : nullptr);
   LCN_CHECK_CUDA(cudaEventRecord(ax->ev_done, ax->st));
-  lcn_launch(k_pack_mid, dim3(dim3(m->nnz * m->FC * m->FC, n_mid)), dim3(256), 0, st, 
-      params, lt, make_pairs(m), m->sup, sc, mask, m->d.F, m->FC, m->nnz,
-      reinterpret_cast<float*>(ws + lay.off_wp32), reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16f),
-      reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16b),
-      x3 ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16f_lo) : nullptr,
-      x3 ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16b_lo) : nullptr,
-      x3 ? 1 : 0 /* fp32 copy: the parity tap of the fp32-parity path (lcn_model_read_tensor kind 2) */, 1,
-      m->mask_off, cmask, m->n_lin, m->d.max_norm, sc, mask);
+  if (n_mid > 0)
+    lcn_launch(k_pack_mid, dim3(dim3(m->nnz * m->FC * m->FC, n_mid)), dim3(256), 0, st,
+        params, lt, make_pairs(m), m->sup, sc, m->d.F, m->FC, m->nnz,
+        x3 ? reinterpret_cast<float*>(ws + lay.off_wp32) : nullptr /* the parity tap (lcn_model_read_tensor kind 2) */,
+        reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16f), reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16b),
+        x3 ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16f_lo) : nullptr,
+        x3 ? reinterpret_cast<__nv_bfloat16*>(ws + lay.off_wp16b_lo) : nullptr,
+        m->mask_off, cmask, m->d.max_norm);
   LCN_CHECK_LAUNCH();
   LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_done, 0));
   return LCN_OK;

@@ -14,9 +14,12 @@ pytestmark = pytest.mark.gpu
 TOL = {"fp32": 1e-4, "bf16": 1e-2}
 
 
-@pytest.mark.parametrize("mask_type,knn", [("locally_connected", 3), ("locally_connected", 1), ("exponential", 2)])
-def test_mask_and_effective_weights(mask_type, knn):
-    eng, cfg, p = make_pair(L=1, knn=knn, mask_type=mask_type)
+@pytest.mark.parametrize("mask_type,knn,L", [("locally_connected", 3, 1), ("locally_connected", 1, 1), ("exponential", 2, 1),
+                                             ("locally_connected", 3, 0), ("exponential", 2, 0)],
+                         ids=["locally_connected-3", "locally_connected-1", "exponential-2", "locally_connected-3-L0",
+                              "exponential-2-L0"])
+def test_mask_and_effective_weights(mask_type, knn, L):
+    eng, cfg, p = make_pair(L=L, knn=knn, mask_type=mask_type)
     eng.prepare()
     mask = O.mask_values(cfg, p)
     got = eng.read_tensor(3, 0, 128, 128).cpu().numpy()
@@ -66,7 +69,7 @@ def _per_layer_check(eng, cfg, p, x, n, bn_group, rate, tol, keep=None):
 
 
 @pytest.mark.parametrize("path", ["fp32", "bf16"])
-@pytest.mark.parametrize("L,knn,n,bn_group", [(1, 3, 200, 200), (2, 2, 300, 128), (1, 3, 256, 256)])
+@pytest.mark.parametrize("L,knn,n,bn_group", [(1, 3, 200, 200), (2, 2, 300, 128), (1, 3, 256, 256), (0, 3, 200, 200)])
 def test_forward_per_layer_and_end_to_end(path, L, knn, n, bn_group):
     eng, cfg, p = make_pair(L=L, knn=knn, path=path)
     x, _ = synth_xy(n)
@@ -164,7 +167,8 @@ GRAD_TOL = {"fp32": 2e-3, "bf16": 1e-1}
 @pytest.mark.parametrize("path", ["fp32", "bf16"])
 @pytest.mark.parametrize("L,knn,mask_type,n,rate", [(1, 3, "locally_connected", 200, 0.0),
                                                      (2, 2, "locally_connected", 256, 0.25),
-                                                     (1, 1, "exponential", 128, 0.0)])
+                                                     (1, 1, "exponential", 128, 0.0),
+                                                     (0, 3, "locally_connected", 200, 0.25)])
 def test_backward_gradients(path, L, knn, mask_type, n, rate):
     eng, cfg, p = make_pair(L=L, knn=knn, mask_type=mask_type, path=path)
     x, y = synth_xy(n)
@@ -186,9 +190,10 @@ def test_backward_gradients(path, L, knn, mask_type, n, rate):
         assert e < tol, f"grad {k}: rel err {e}"
 
 
-@pytest.mark.parametrize("path", ["fp32", "bf16"])
-def test_train_steps_match_tf1_adam(path):
-    eng, cfg, p = make_pair(L=1, knn=3, path=path, perturb=True)
+@pytest.mark.parametrize("path,L", [("fp32", 1), ("bf16", 1), ("fp32", 0), ("bf16", 0)],
+                         ids=["fp32", "bf16", "fp32-L0", "bf16-L0"])
+def test_train_steps_match_tf1_adam(path, L):
+    eng, cfg, p = make_pair(L=L, knn=3, path=path, perturb=True)
     n = 256
     x, y = synth_xy(n)
     xd, yd = dev(x), dev(y)
