@@ -302,7 +302,7 @@ WsLayout lcn_ws_layout(const lcn_model* m, int64_t n_rows, int bn_group, int tra
   w.off_d = take(act * w.n_d);
   w.off_dz = take(training ? 2 * act : 0);
   w.off_dbpart = take(training ? sizeof(float) * (size_t)m->n_bn * 2 * m->sm_count * P : 0);
-  w.off_keep = take(training ? (size_t)m->n_bn * w.rows_pad * (P / 8) : 0);
+  w.off_keep = take(training ? sizeof(uint16_t) * (size_t)m->n_bn * w.rows_pad * (P / 8) : 0);
   w.off_stack = take(w.fused ? lcn_stack_scratch_bytes(m, bn_group) : 0);
   w.total = off;
   return w;

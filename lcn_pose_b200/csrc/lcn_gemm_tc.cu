@@ -1077,6 +1077,16 @@ extern "C" int lcn_debug_tcw_units(const uint32_t* row17, int FCK, int FCN, int 
   return p.n_units;
 }
 
+// dynamic shared memory of a k_tc_wgrad CTA: the operand ring, plus the alignment slack of its 1024-byte base
+static inline size_t tcw_smem_bytes() { return (size_t)TCW_STAGES * TCW_STAGE_BYTES + 1024; }
+
+int lcn_tc_wgrad_footprint(bool x3, cudaFuncAttributes* attr, size_t* dyn_smem, int* threads) {
+  LCN_CHECK_CUDA(x3 ? cudaFuncGetAttributes(attr, k_tc_wgrad<true>) : cudaFuncGetAttributes(attr, k_tc_wgrad<false>));
+  *dyn_smem = tcw_smem_bytes();
+  *threads = TCW_THREADS;
+  return LCN_OK;
+}
+
 static int launch_tc_wgrad(TcwParams& p, const __nv_bfloat16* A, const __nv_bfloat16* dZ, float* dW, int tiles,
                            int sm_count, cudaStream_t st, bool x3 = false) {
   tcw_build_units(p);
@@ -1089,7 +1099,7 @@ static int launch_tc_wgrad(TcwParams& p, const __nv_bfloat16* A, const __nv_bflo
   while (tpc < tiles && (long)units * ((tiles + tpc - 1) / tpc) > slots) ++tpc;
   p.tiles_per_cta = tpc;
   int splits = (tiles + tpc - 1) / tpc;
-  size_t smem = (size_t)TCW_STAGES * TCW_STAGE_BYTES + 1024;
+  const size_t smem = tcw_smem_bytes();
   static std::once_flag once;
   static cudaError_t rc = cudaSuccess;
   std::call_once(once, [smem] {

@@ -134,7 +134,7 @@ struct WsLayout {
   size_t off_d, d_stride; int n_d;   // gradient ping-pong buffers (training)
   size_t off_dz;                     // dZ buffers (training): layer l uses buffer l & 1 (wgrad of l overlaps BN backward of l-1)
   size_t off_dbpart;                 // float[n_bn][2*SMs][P] per-block bias-gradient partial rows (training)
-  size_t off_keep;                   // uint8[n_bn][rows_pad][P/8] dropout keep bits (training)
+  size_t off_keep;                   // uint16[n_bn][rows_pad][P/8] dropout keep bits | LeakyReLU sign bits << 8 (training)
   int fused;                         // inference runs as the fused cluster kernel (lcn_stack_tc.cu)
   size_t off_stack;                  // its per-cluster L2-resident activation scratch
   size_t total;
@@ -347,6 +347,9 @@ int lcn_tc_gemm(const lcn_model* m, const WsLayout& lay, int mid_index, int tran
                 const char* wpacked_lo = nullptr);
 int lcn_tc_wgrad(const lcn_model* m, const WsLayout& lay, const __nv_bfloat16* A, const __nv_bfloat16* dZ,
                  float* dW /* dense [P,P] */, cudaStream_t st, bool x3 = false);
+// what one k_tc_wgrad CTA (x3: the split-bf16 instantiation) occupies on an SM: attributes, launched dynamic shared
+// memory, threads
+int lcn_tc_wgrad_footprint(bool x3, cudaFuncAttributes* attr, size_t* dyn_smem, int* threads);
 int lcn_tc_head(const lcn_model* m, const WsLayout& lay, const __nv_bfloat16* A, const char* wpacked,
                 const float* bias, const float* x, float* out_user, float* out_ws, cudaStream_t st);
 int lcn_tc_head_dgrad(const lcn_model* m, const WsLayout& lay, const __nv_bfloat16* dOut16, const char* wpacked,

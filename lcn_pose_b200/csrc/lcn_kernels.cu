@@ -526,15 +526,16 @@ __global__ void __launch_bounds__(256) k_bn_finalize(const float* __restrict__ p
 // Persistent: grid = 2 x SMs blocks of (P/8, Y) threads, each block owns a contiguous range of rows; a thread
 // owns 8 consecutive columns (16 B of bf16) and walks the rows with a register double buffer (the loads of
 // row r+Y are in flight while row r is processed).  Per-channel scale/shift live in shared memory and are
-// reloaded when the row range crosses into the next BatchNorm group.  When dropout is active the keep
-// decisions are also written as one byte per (row, 8 columns) so that backward does not redraw Philox.
+// reloaded when the row range crosses into the next BatchNorm group.  In training, per (row, 8 columns) the keep
+// decisions (low byte: backward does not redraw Philox) and the signs ybn > 0 of the LeakyReLU (high byte: backward
+// takes the branch the forward took without forming ybn again) are written as one uint16.
 // ------------------------------------------------------------------------------------------------
 #define EW_MAXT 288   // (P/8) x Y threads: (136,2) for F=64, (272,1) for F=128
 template <typename T>
 __global__ void __launch_bounds__(EW_MAXT, 2) k_bn_act(const T* __restrict__ Z, const float* __restrict__ stat,
                                                        const float* __restrict__ gamma, const float* __restrict__ beta,
                                                        const T* __restrict__ res, T* __restrict__ Aout,
-                                                       uint8_t* __restrict__ keepbits, int P, int F, int rows_pad,
+                                                       uint16_t* __restrict__ keepbits, int P, int F, int rows_pad,
                                                        int bn_group, int gstride, float rate, uint64_t seed,
                                                        uint64_t step, int layer, const lcn_step_scalars* __restrict__ dyn) {
   lcn_pdl_prologue();
@@ -604,6 +605,7 @@ __global__ void __launch_bounds__(EW_MAXT, 2) k_bn_act(const T* __restrict__ Z, 
 #pragma unroll
         for (int q = 0; q < 8; ++q) {
           float v = fmaf(zc[q], sc[q], sh[q]);
+          if (v > 0.f) kb |= 0x100u << q;
           v = v > 0.f ? v : LCN_LRELU * v;
           v = ((kb >> q) & 1u) ? v * inv_keep : 0.f;
           if (res != nullptr) v += rc[q];
@@ -611,7 +613,7 @@ __global__ void __launch_bounds__(EW_MAXT, 2) k_bn_act(const T* __restrict__ Z, 
         }
       }
       lcn_st8(Aout, oc, y);
-      if (keepbits != nullptr && rate > 0.f) keepbits[(size_t)r * (P >> 3) + threadIdx.x] = (uint8_t)kb;
+      if (keepbits != nullptr) keepbits[(size_t)r * (P >> 3) + threadIdx.x] = (uint16_t)kb;
     }
 #pragma unroll
     for (int q = 0; q < 8; ++q) {
@@ -634,7 +636,7 @@ __global__ void __launch_bounds__(EW_MAXT, 2) k_bn_act_pre(const __nv_bfloat16* 
                                                            const float* __restrict__ beta,
                                                            const __nv_bfloat16* __restrict__ res,
                                                            __nv_bfloat16* __restrict__ Aout,
-                                                           uint8_t* __restrict__ keepbits, int P, int F, int rows_pad,
+                                                           uint16_t* __restrict__ keepbits, int P, int F, int rows_pad,
                                                            int bn_group, float rate, uint64_t seed, uint64_t step,
                                                            int layer, const lcn_step_scalars* __restrict__ dyn,
                                                            const double* __restrict__ gacc, float* __restrict__ stat_out,
@@ -719,6 +721,7 @@ __global__ void __launch_bounds__(EW_MAXT, 2) k_bn_act_pre(const __nv_bfloat16* 
         for (int h = 0; h < 2; ++h) {
           const int q = 2 * e + h;
           float v = fmaf(h ? z2.y : z2.x, sc[q], sh[q]);
+          if (v > 0.f) kb |= 0x100u << q;
           v = v > 0.f ? v : LCN_LRELU * v;
           v = ((kb >> q) & 1u) ? v * inv_keep : 0.f;
           if (res != nullptr) v += h ? r2.y : r2.x;
@@ -727,7 +730,7 @@ __global__ void __launch_bounds__(EW_MAXT, 2) k_bn_act_pre(const __nv_bfloat16* 
       }
     }
     lcn_st8(Aout, lcn_off<__nv_bfloat16>(r, c8, P), y);
-    if (keepbits != nullptr && rate > 0.f) keepbits[(size_t)r * (P >> 3) + threadIdx.x] = (uint8_t)kb;
+    if (keepbits != nullptr) keepbits[(size_t)r * (P >> 3) + threadIdx.x] = (uint16_t)kb;
   }
 }
 
@@ -891,192 +894,232 @@ __global__ void __launch_bounds__(256) k_last_layer_bwd(const T* __restrict__ A,
 
 // ------------------------------------------------------------------------------------------------
 // BN / LeakyReLU / dropout backward (training = one group).
-//   dy   = dOut * keep/(1-rate) * (ybn > 0 ? 1 : 0.2)
-//   sums = (sum dy, sum dy*xhat) per channel        [k_bn_bwd_reduce]
-//   dZ   = gamma*rstd*(dy - s1/n - xhat*s2/n)       [k_bn_bwd_apply], db = sum_rows dZ
-// Persistent like k_bn_act: grid = 2 x SMs blocks of (P/8, Y) threads, strided rows, register double buffer;
-// keep decisions come from the bits written by k_bn_act; one block-level reduction, then one atomic per
-// channel (reduce) / per column (apply) per block.
+//   dy   = dOut * keep/(1-rate) * (ybn > 0 ? 1 : 0.2),  keep and ybn > 0 as stored by k_bn_act(_pre)
+//   sums = (sum dy, rstd * sum dy*(z - mean)) = (sum dy, sum dy*xhat) per channel   [k_bn_bwd_reduce]
+//   dZ   = sc*(dy - s1/n - xhat*s2/n) = sc*dy + alpha + beta*z                     [k_bn_bwd_apply], db = sum_rows dZ
+// Persistent like k_bn_act: grid = 2 x SMs blocks of (P/8, Y) threads, strided rows, a register double buffer of the
+// rows as loaded (Raw8); keep decisions and LeakyReLU branches come from the bits written by k_bn_act(_pre), so neither
+// kernel forms ybn; one block-level reduction, then one atomic per channel (reduce) / one partial row (apply) per block.
+//
+// Both kernels run while the weight-gradient GEMM of the layer before (k_tc_wgrad, one 224-thread CTA with ~195 KB of
+// shared memory and 72 registers per thread on 124 of the SMs) is still running on the side stream.  Their grid
+// assumes two blocks per SM, so two blocks must fit BESIDE that CTA (else 124 of 296 run as a second wave): at most
+// 72 registers per thread (register files are per SM sub-partition: 16 K registers, 2 wgrad warps + 5 of these warps
+// in each), the per-channel constants in shared memory rather than registers, <= 15 KB of shared memory per block,
+// and the maximum shared-memory carveout (backward_impl).  lcn_debug_bn_bwd_fit reports the fit for the device.
 // ------------------------------------------------------------------------------------------------
-struct BnConsts {
-  float sc[8], sh[8], rstd[8], mr[8];   // scale, shift, rstd, mean*rstd for the thread's 8 channels
-};
-__device__ __forceinline__ void bn_bwd_dy8(const float z[8], const float d[8], uint32_t kb, const BnConsts& k,
-                                           float inv_keep, float dy[8], float xh[8]) {
-#pragma unroll
-  for (int q = 0; q < 8; ++q) {
-    float ybn = fmaf(z[q], k.sc[q], k.sh[q]);
-    float v = ((kb >> q) & 1u) ? d[q] * inv_keep : 0.f;
-    dy[q] = ybn > 0.f ? v : LCN_LRELU * v;
-    xh[q] = fmaf(z[q], k.rstd[q], -k.mr[q]);
-  }
+#define LCN_BN_BWD_MAXREG 72
+
+// one thread's 8 consecutive elements of a row, as loaded: 16 B per bf16 plane (4 registers for bf16, 8 for split
+// bf16 instead of 8 floats); at(q) is what lcn_ld8 would have produced for element q
+template <typename T>
+struct Raw8;
+__device__ __forceinline__ float bf16_word_at(const uint4& u, int q) {
+  const uint32_t w = q < 2 ? u.x : q < 4 ? u.y : q < 6 ? u.z : u.w;
+  return __uint_as_float((q & 1) ? (w & 0xffff0000u) : (w << 16));
 }
-__device__ __forceinline__ void bn_load_consts(const float* stat, const float* gamma, const float* beta, int F,
-                                               int f0, float* s_a, float* s_b, float* s_c, float* s_d, BnConsts& k) {
-  int tid = threadIdx.y * blockDim.x + threadIdx.x;
-  if (tid < F) {
-    float mean = stat[tid * 2], rstd = stat[tid * 2 + 1];
-    float sc = gamma[tid] * rstd;
-    s_a[tid] = sc;
-    s_b[tid] = beta[tid] - mean * sc;
-    s_c[tid] = rstd;
-    s_d[tid] = mean * rstd;
+template <>
+struct Raw8<__nv_bfloat16> {
+  uint4 h;
+  __device__ __forceinline__ void load(const __nv_bfloat16* p, size_t i) { h = *reinterpret_cast<const uint4*>(p + i); }
+  __device__ __forceinline__ float at(int q) const { return bf16_word_at(h, q); }
+};
+template <>
+struct Raw8<lcn_sp16> {
+  uint4 h, l;
+  __device__ __forceinline__ void load(const lcn_sp16* p, size_t i) {
+    const __nv_bfloat16* q = reinterpret_cast<const __nv_bfloat16*>(p);
+    h = *reinterpret_cast<const uint4*>(q + i);
+    l = *reinterpret_cast<const uint4*>(q + i + LCN_SP_LO);
   }
-  __syncthreads();
-#pragma unroll
-  for (int q = 0; q < 8; ++q) {
-    k.sc[q] = s_a[f0 + q];
-    k.sh[q] = s_b[f0 + q];
-    k.rstd[q] = s_c[f0 + q];
-    k.mr[q] = s_d[f0 + q];
-  }
+  __device__ __forceinline__ float at(int q) const { return bf16_word_at(h, q) + bf16_word_at(l, q); }
+};
+
+// Per-channel constants of the backward kernels: s_k[k][f] in shared memory.  lds<W>(s_f0, k, h, v) reads constants k
+// of the thread's channels f0 + h .. f0 + h + W - 1, s_f0 being the shared address of s_k[0][f0].  volatile: read again
+// for every row, where they are used, instead of hoisted out of the row loop into live registers.
+#define BN_BWD_KSTRIDE 256
+template <int W>
+__device__ __forceinline__ void lds(uint32_t s_f0, int k, int h, float v[W]) {
+  static_assert(W == 2 || W == 4, "2 or 4 channels");
+  const uint32_t a = s_f0 + (uint32_t)(k * BN_BWD_KSTRIDE + h) * 4u;
+  if constexpr (W == 4)
+    asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v[0]), "=f"(v[1]), "=f"(v[2]), "=f"(v[3]) : "r"(a));
+  else
+    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v[0]), "=f"(v[1]) : "r"(a));
+}
+
+// dy of element q: its dropout keep bit (bit q) and the LeakyReLU branch the forward pass took (bit 8 + q), both as
+// k_bn_act(_pre) wrote them
+__device__ __forceinline__ float bn_bwd_dy(float d, uint32_t kb, int q, float inv_keep) {
+  const float v = ((kb >> q) & 1u) ? d * inv_keep : 0.f;
+  return ((kb >> (8 + q)) & 1u) ? v : LCN_LRELU * v;
 }
 
 template <typename T>
-__global__ void __launch_bounds__(EW_MAXT, 2) k_bn_bwd_reduce(const T* __restrict__ dOut, const T* __restrict__ Z,
-                                                              const uint8_t* __restrict__ keepbits,
-                                                              const float* __restrict__ stat,
-                                                              const float* __restrict__ gamma,
-                                                              const float* __restrict__ beta, float* __restrict__ sums,
-                                                              int P, int F, int bn_group, float rate) {
+__global__ void __maxnreg__(LCN_BN_BWD_MAXREG) k_bn_bwd_reduce(const T* __restrict__ dOut, const T* __restrict__ Z,
+                                                               const uint16_t* __restrict__ keepbits,
+                                                               const float* __restrict__ stat, float* __restrict__ sums,
+                                                               int P, int F, int bn_group, float rate) {
   lcn_pdl_prologue();
-  extern __shared__ __align__(16) float red[];   // [Y][P/8][16]
-  __shared__ __align__(16) float s_a[256], s_b[256], s_c[256], s_d[256];
+  __shared__ __align__(16) float s_k[1][BN_BWD_KSTRIDE];    // mean
+  extern __shared__ float red[];                 // [warps][16 values][F/8 octets]: warp sums of (dy, dy*(z - mean))
   const int Y = blockDim.y, c8 = threadIdx.x * 8, f0 = c8 % F;
-  BnConsts k;
-  bn_load_consts(stat, gamma, beta, F, f0, s_a, s_b, s_c, s_d, k);
-  float inv_keep = rate > 0.f ? 1.f / (1.f - rate) : 1.f;
+  const int nt = blockDim.x * Y, tid = threadIdx.y * blockDim.x + threadIdx.x;
+  if (tid < F) s_k[0][tid] = stat[tid * 2];
+  __syncthreads();
+  const uint32_t s_f0 = (uint32_t)__cvta_generic_to_shared(&s_k[0][f0]);
+  const float inv_keep = rate > 0.f ? 1.f / (1.f - rate) : 1.f;
   float s1[8], s2[8];
 #pragma unroll
   for (int q = 0; q < 8; ++q) s1[q] = s2[q] = 0.f;
   const int stride = gridDim.x * Y;
   int r = blockIdx.x * Y + threadIdx.y;
-  float zc[8], dc[8], zn[8], dn[8];
-  uint32_t kc = 0xffu, kn = 0xffu;
+  Raw8<T> zc, dc, zn, dn;
+  uint32_t kc = 0u, kn = 0u;
   if (r < bn_group) {
-    size_t o = lcn_off<T>(r, c8, P);
-    lcn_ld8(Z, o, zc);
-    lcn_ld8(dOut, o, dc);
-    if (rate > 0.f) kc = keepbits[(size_t)r * (P >> 3) + threadIdx.x];
+    const size_t o = lcn_off<T>(r, c8, P);
+    zc.load(Z, o);
+    dc.load(dOut, o);
+    kc = keepbits[(size_t)r * (P >> 3) + threadIdx.x];
   }
   for (; r < bn_group; r += stride) {
-    int rn = r + stride;
+    const int rn = r + stride;
     if (rn < bn_group) {
-      size_t o = lcn_off<T>(rn, c8, P);
-      lcn_ld8(Z, o, zn);
-      lcn_ld8(dOut, o, dn);
-      if (rate > 0.f) kn = keepbits[(size_t)rn * (P >> 3) + threadIdx.x];
+      const size_t o = lcn_off<T>(rn, c8, P);
+      zn.load(Z, o);
+      dn.load(dOut, o);
+      kn = keepbits[(size_t)rn * (P >> 3) + threadIdx.x];
     }
-    float dy[8], xh[8];
-    bn_bwd_dy8(zc, dc, kc, k, inv_keep, dy, xh);
 #pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      s1[q] += dy[q];
-      s2[q] = fmaf(dy[q], xh[q], s2[q]);
-      zc[q] = zn[q];
-      dc[q] = dn[q];
+    for (int h = 0; h < 8; h += 4) {             // the means of 4 channels are live at a time
+      float mu[4];
+      lds<4>(s_f0, 0, h, mu);
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const int q = h + e;
+        const float dy = bn_bwd_dy(dc.at(q), kc, q, inv_keep);
+        s1[q] += dy;
+        s2[q] = fmaf(dy, zc.at(q) - mu[e], s2[q]);
+      }
     }
+    zc = zn;
+    dc = dn;
     kc = kn;
   }
-  int nt = blockDim.x;
-  float* mine = red + ((size_t)threadIdx.y * nt + threadIdx.x) * 16;
+  // Threads tid, tid ^ F/8, ... of a warp hold the same channel octet (tid % (F/8); F/8 divides 32 and the row length
+  // P/8): butterfly over them (the partial last warp has 16 lanes), then lanes 0 .. F/8-1 store the warp's sums and
+  // 2F threads add up the warps (plain stores: shared-memory float atomics are compare-and-swap loops that the 9 warps
+  // of a block, arriving together, serialise on)
+  const int lane = tid & 31, per = F / 8, nv = min(32, nt - (tid & ~31));
+  const unsigned mask = nv == 32 ? 0xffffffffu : (1u << nv) - 1u;
+  for (int off = per; off < nv; off <<= 1) {
 #pragma unroll
-  for (int q = 0; q < 8; ++q) {
-    mine[q] = s1[q];
-    mine[8 + q] = s2[q];
+    for (int q = 0; q < 8; ++q) {
+      s1[q] += __shfl_xor_sync(mask, s1[q], off);
+      s2[q] += __shfl_xor_sync(mask, s2[q], off);
+    }
+  }
+  if (lane < per) {
+    float* mine = red + (tid >> 5) * 2 * F + lane;
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+      mine[q * per] = s1[q];
+      mine[(8 + q) * per] = s2[q];
+    }
   }
   __syncthreads();
-  int per = F / 8;                               // threads (x) per joint
-  int t = threadIdx.y * nt + threadIdx.x;
-  if (t < per * 16) {                            // one thread per (channel octet, value)
-    int oct = t / 16, v = t % 16;
+  const int nw = (nt + 31) >> 5;
+  for (int i = tid; i < 2 * F; i += nt) {
     float a = 0.f;
-    for (int y = 0; y < Y; ++y)
-      for (int j = 0; j < LCN_J; ++j) a += red[((size_t)y * nt + oct + j * per) * 16 + v];
-    int f = oct * 8 + (v & 7);
-    atomicAdd(&sums[f * 2 + (v >> 3)], a);
+    for (int w = 0; w < nw; ++w) a += red[w * 2 * F + i];
+    const int v = i / per, f = (i % per) * 8 + (v & 7);
+    atomicAdd(&sums[f * 2 + (v >> 3)], v < 8 ? a : a * stat[f * 2 + 1]);
   }
 }
 
 template <typename T, bool kSync>
-__global__ void __launch_bounds__(EW_MAXT, 2) k_bn_bwd_apply(const T* __restrict__ dOut, const T* __restrict__ Z,
-                                                             const uint8_t* __restrict__ keepbits,
-                                                             const float* __restrict__ stat,
-                                                             const float* __restrict__ gamma,
-                                                             const float* __restrict__ beta,
-                                                             const float* __restrict__ sums, T* __restrict__ dZ,
-                                                             float* __restrict__ dbpart, float* __restrict__ dgamma,
-                                                             float* __restrict__ dbeta, int P, int F, int rows_pad,
-                                                             int bn_group, float rate, const float* __restrict__ gmean) {
+__global__ void __maxnreg__(LCN_BN_BWD_MAXREG) k_bn_bwd_apply(const T* __restrict__ dOut, const T* __restrict__ Z,
+                                                              const uint16_t* __restrict__ keepbits,
+                                                              const float* __restrict__ stat,
+                                                              const float* __restrict__ gamma,
+                                                              const float* __restrict__ sums, T* __restrict__ dZ,
+                                                              float* __restrict__ dbpart, float* __restrict__ dgamma,
+                                                              float* __restrict__ dbeta, int P, int F, int rows_pad,
+                                                              int bn_group, float rate, const float* __restrict__ gmean) {
   lcn_pdl_prologue();
   extern __shared__ __align__(16) float red[];   // [Y-1][P] column sums of the other row-threads
-  __shared__ __align__(16) float s_a[256], s_b[256], s_c[256], s_d[256];
+  __shared__ __align__(16) float s_k[3][BN_BWD_KSTRIDE];    // sc, alpha, beta
   const int Y = blockDim.y, c8 = threadIdx.x * 8, f0 = c8 % F;
-  BnConsts k;
-  bn_load_consts(stat, gamma, beta, F, f0, s_a, s_b, s_c, s_d, k);
-  float m1[8], m2[8];
-  if constexpr (kSync) {         // synchronised BatchNorm: (S1, S2) / N over all ranks' rows, from k_bn_sync
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      m1[q] = gmean[(f0 + q) * 2];
-      m2[q] = gmean[(f0 + q) * 2 + 1];
+  const int tid = threadIdx.y * blockDim.x + threadIdx.x;
+  if (tid < F) {
+    const float mean = stat[tid * 2], rstd = stat[tid * 2 + 1];
+    const float sc = gamma[tid] * rstd;
+    float m1, m2;
+    if constexpr (kSync) {       // synchronised BatchNorm: (S1, S2) / N over all ranks' rows, from k_bn_sync
+      m1 = gmean[tid * 2];
+      m2 = gmean[tid * 2 + 1];
+    } else {
+      const float inv_n = 1.f / ((float)bn_group * (float)LCN_J);
+      m1 = sums[tid * 2] * inv_n;
+      m2 = sums[tid * 2 + 1] * inv_n;
     }
-  } else {
-    float inv_n = 1.f / ((float)bn_group * (float)LCN_J);
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      m1[q] = sums[(f0 + q) * 2] * inv_n;
-      m2[q] = sums[(f0 + q) * 2 + 1] * inv_n;
-    }
-  }
-  if (blockIdx.x == 0 && threadIdx.y == 0 && (int)threadIdx.x < F / 8) {
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      dbeta[f0 + q] = sums[(f0 + q) * 2];
-      dgamma[f0 + q] = sums[(f0 + q) * 2 + 1];
+    s_k[0][tid] = sc;
+    // sc*(dy - m1 - xhat*m2) with xhat = z*rstd - mean*rstd
+    s_k[1][tid] = sc * (m2 * (mean * rstd) - m1);
+    s_k[2][tid] = -(sc * m2) * rstd;
+    if (blockIdx.x == 0) {
+      dbeta[tid] = sums[tid * 2];
+      dgamma[tid] = sums[tid * 2 + 1];
     }
   }
-  float inv_keep = rate > 0.f ? 1.f / (1.f - rate) : 1.f;
+  __syncthreads();
+  const uint32_t s_f0 = (uint32_t)__cvta_generic_to_shared(&s_k[0][f0]);
+  const float inv_keep = rate > 0.f ? 1.f / (1.f - rate) : 1.f;
   float bsum[8];
 #pragma unroll
   for (int q = 0; q < 8; ++q) bsum[q] = 0.f;
   const int stride = gridDim.x * Y;
   int r = blockIdx.x * Y + threadIdx.y;
-  float zc[8], dc[8], zn[8], dn[8];
-  uint32_t kc = 0xffu, kn = 0xffu;
+  Raw8<T> zc, dc, zn, dn;
+  uint32_t kc = 0u, kn = 0u;
   if (r < bn_group) {
-    size_t o = lcn_off<T>(r, c8, P);
-    lcn_ld8(Z, o, zc);
-    lcn_ld8(dOut, o, dc);
-    if (rate > 0.f) kc = keepbits[(size_t)r * (P >> 3) + threadIdx.x];
+    const size_t o = lcn_off<T>(r, c8, P);
+    zc.load(Z, o);
+    dc.load(dOut, o);
+    kc = keepbits[(size_t)r * (P >> 3) + threadIdx.x];
   }
   for (; r < rows_pad; r += stride) {
-    int rn = r + stride;
+    const int rn = r + stride;
     if (rn < bn_group) {
-      size_t o = lcn_off<T>(rn, c8, P);
-      lcn_ld8(Z, o, zn);
-      lcn_ld8(dOut, o, dn);
-      if (rate > 0.f) kn = keepbits[(size_t)rn * (P >> 3) + threadIdx.x];
+      const size_t o = lcn_off<T>(rn, c8, P);
+      zn.load(Z, o);
+      dn.load(dOut, o);
+      kn = keepbits[(size_t)rn * (P >> 3) + threadIdx.x];
     }
     float dz[8];
     if (r >= bn_group) {                          // tile padding rows: dZ must be zero (wgrad reduces over rows)
 #pragma unroll
       for (int q = 0; q < 8; ++q) dz[q] = 0.f;
     } else {
-      float dy[8], xh[8];
-      bn_bwd_dy8(zc, dc, kc, k, inv_keep, dy, xh);
 #pragma unroll
-      for (int q = 0; q < 8; ++q) {
-        dz[q] = k.sc[q] * (dy[q] - m1[q] - xh[q] * m2[q]);
-        bsum[q] += dz[q];
+      for (int h = 0; h < 8; h += 4) {           // the constants of 4 channels are live at a time
+        float sc[4], al[4], be[4];
+        lds<4>(s_f0, 0, h, sc);
+        lds<4>(s_f0, 1, h, al);
+        lds<4>(s_f0, 2, h, be);
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          const int q = h + e;
+          const float dy = bn_bwd_dy(dc.at(q), kc, q, inv_keep);
+          dz[q] = fmaf(sc[e], dy, fmaf(be[e], zc.at(q), al[e]));
+          bsum[q] += dz[q];
+        }
       }
     }
     lcn_st8(dZ, lcn_off<T>(r, c8, P), dz);
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      zc[q] = zn[q];
-      dc[q] = dn[q];
-    }
+    zc = zn;
+    dc = dn;
     kc = kn;
   }
   // db: combine the row-threads of a column octet in shared memory; one partial row per block (no atomics:
@@ -1432,11 +1475,18 @@ static inline float* bn_stat(char* ws, const WsLayout& lay, const lcn_model* m, 
 struct EwGeom {
   int ewy, grid, rows_thr;
 };
+static inline int ew_rows_per_block(int P) { return (P / 8) * 2 <= EW_MAXT ? 2 : 1; }
 static inline EwGeom ew_geom(const lcn_model* m, const WsLayout& lay) {
-  const int ewy = (m->P / 8) * 2 <= EW_MAXT ? 2 : 1;
+  const int ewy = ew_rows_per_block(m->P);
   const int grid = (int)std::min<int64_t>(2 * m->sm_count, lay.rows_pad / ewy);
   return {ewy, grid, (int)((lay.rows_pad / ewy + grid - 1) / grid)};
 }
+// dynamic shared memory of k_bn_bwd_reduce: 2F warp sums per warp; of k_bn_bwd_apply: the column sums of the
+// row-threads 1 .. ewy-1
+static inline size_t bn_bwd_reduce_smem(int P, int ewy) {
+  return (size_t)((P / 8 * ewy + 31) / 32) * 2 * (P / LCN_J) * sizeof(float);
+}
+static inline size_t bn_bwd_apply_smem(int P, int ewy) { return (size_t)(ewy - 1) * P * sizeof(float); }
 // packed bf16 blocks of mid layer l: forward (Y = A*Wm) or transposed (dA = dZ*Wm^T); lo: their lo parts on the
 // split-bf16 path, nullptr on the bf16 path
 struct MidWeights {
@@ -1526,9 +1576,8 @@ static int forward_impl(const FwdArgs& a) {
       gacc = nullptr;                  // k_bn_act_pre reads the global statistics from stat
     }
     const T* res = L.res_from >= 0 ? reinterpret_cast<const T*>(a_buf(ws, lay, L.res_from)) : nullptr;
-    uint8_t* keepbits = (lay.training && a.dropout_rate > 0.f)
-                            ? reinterpret_cast<uint8_t*>(ws + lay.off_keep) + (size_t)l * lay.rows_pad * (P / 8)
-                            : nullptr;
+    uint16_t* keepbits = lay.training ? reinterpret_cast<uint16_t*>(ws + lay.off_keep) + (size_t)l * lay.rows_pad * (P / 8)
+                                      : nullptr;
     if (pre)
       lcn_launch(k_bn_act_pre, dim3(ew.grid), dim3(P / 8, ew.ewy), 0, st, reinterpret_cast<const __nv_bfloat16*>(Z), stat,
                  a.params + L.gamma_off, a.params + L.beta_off, reinterpret_cast<const __nv_bfloat16*>(res),
@@ -1627,21 +1676,33 @@ static int backward_impl(const lcn_model* m, const float* params, char* ws, cons
     LCN_CHECK_LAUNCH();
   }
   const EwGeom ew = ew_geom(m, lay);
-  size_t red_smem = (size_t)ew.ewy * (P / 8) * 16 * sizeof(float);
+  // the weight-gradient GEMM beside these kernels needs the SM's full shared-memory carveout; an SM that holds only
+  // BatchNorm blocks keeps that configuration, so a weight-gradient CTA can still join them
+  static std::once_flag carveout_once;
+  static cudaError_t carveout_rc = cudaSuccess;
+  std::call_once(carveout_once, [] {
+    const int c = cudaSharedmemCarveoutMaxShared;
+    carveout_rc = cudaFuncSetAttribute(k_bn_bwd_reduce<T>, cudaFuncAttributePreferredSharedMemoryCarveout, c);
+    if (carveout_rc == cudaSuccess)
+      carveout_rc = cudaFuncSetAttribute(k_bn_bwd_apply<T, false>, cudaFuncAttributePreferredSharedMemoryCarveout, c);
+    if (carveout_rc == cudaSuccess)
+      carveout_rc = cudaFuncSetAttribute(k_bn_bwd_apply<T, true>, cudaFuncAttributePreferredSharedMemoryCarveout, c);
+  });
+  LCN_CHECK_CUDA(carveout_rc);
   LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_ms, 0));   // the bucket is clear before this stream stores into it
   for (int l = m->n_bn - 1; l >= 0; --l) {
     const LayerInfo& L = m->L[l];
     const T* Z = reinterpret_cast<const T*>(z_buf(ws, lay, l));
     const float* stat = bn_stat(ws, lay, m, l);
     float* sums = reinterpret_cast<float*>(ws + lay.off_bnsum) + (size_t)l * F * 2;
-    const uint8_t* keepbits = reinterpret_cast<const uint8_t*>(ws + lay.off_keep) + (size_t)l * lay.rows_pad * (P / 8);
+    const uint16_t* keepbits = reinterpret_cast<const uint16_t*>(ws + lay.off_keep) + (size_t)l * lay.rows_pad * (P / 8);
     T* dZ = dZbuf(l);
     if (wg_pending[l & 1]) {         // the weight gradient of layer l+2 has read this dZ buffer
       LCN_CHECK_CUDA(cudaStreamWaitEvent(st, ax->ev_wg[l & 1], 0));
       wg_pending[l & 1] = false;
     }
-    lcn_launch(k_bn_bwd_reduce<T>, dim3(ew.grid), dim3(dim3(P / 8, ew.ewy)), red_smem, st, D(cur), Z, keepbits, stat, params + L.gamma_off,
-                                                             params + L.beta_off, sums, P, F, lay.bn_group, rate);
+    lcn_launch(k_bn_bwd_reduce<T>, dim3(ew.grid), dim3(dim3(P / 8, ew.ewy)), bn_bwd_reduce_smem(P, ew.ewy), st, D(cur), Z, keepbits, stat, sums, P, F,
+                                                             lay.bn_group, rate);
     float* gmean = nullptr;            // synchronised BatchNorm: (S1, S2) / N of all ranks, in the layer's accumulator area
     if (bn_sync) {
       LCN_CHECK_LAUNCH();
@@ -1649,8 +1710,8 @@ static int backward_impl(const lcn_model* m, const float* params, char* ws, cons
       rc = lcn_bn_sync(m, m->n_bn + l, LCN_BN_SYNC_SUMS, sums, gmean, lay.n_rows, st);
       if (rc) return rc;
     }
-    lcn_launch(bn_sync ? k_bn_bwd_apply<T, true> : k_bn_bwd_apply<T, false>, dim3(ew.grid), dim3(dim3(P / 8, ew.ewy)), (size_t)ew.ewy * P * sizeof(float), st,
-        D(cur), Z, keepbits, stat, params + L.gamma_off, params + L.beta_off, sums, dZ,
+    lcn_launch(bn_sync ? k_bn_bwd_apply<T, true> : k_bn_bwd_apply<T, false>, dim3(ew.grid), dim3(dim3(P / 8, ew.ewy)), bn_bwd_apply_smem(P, ew.ewy), st,
+        D(cur), Z, keepbits, stat, params + L.gamma_off, sums, dZ,
         reinterpret_cast<float*>(ws + lay.off_dbpart) + (size_t)l * ew.grid * P, graw + L.gamma_off, graw + L.beta_off, P, F, (int)lay.rows_pad, lay.bn_group, rate,
         gmean);
     LCN_CHECK_LAUNCH();
@@ -1711,6 +1772,55 @@ int lcn_launch_backward(const lcn_model* m, const float* params, char* ws, const
   return m->d.path == LCN_PATH_BF16
              ? backward_impl<__nv_bfloat16>(m, params, ws, lay, x, labels, dropout_rate, seed, step, loss, grads_raw, st)
              : backward_impl<lcn_sp16>(m, params, ws, lay, x, labels, dropout_rate, seed, step, loss, grads_raw, st);
+}
+
+// Blocks of each backward BatchNorm kernel that fit on one SM of this device beside one k_tc_wgrad CTA, at the block
+// shape and dynamic shared memory backward_impl launches them with for feature width F.  blocks_out[6]:
+// k_bn_bwd_reduce, k_bn_bwd_apply<false>, k_bn_bwd_apply<true> on the bf16 path (beside k_tc_wgrad<false>), then the
+// same three on the split-bf16 path (beside k_tc_wgrad<true>).  Registers are counted per SM sub-partition, as the CUDA
+// occupancy calculator counts them, and every sub-partition is charged as many k_tc_wgrad warps as the fullest one
+// holds (2 of its 7).  Shared memory is the SM's maximum: the carveout both kernels prefer (backward_impl) and the one
+// the k_tc_wgrad CTA needs.
+extern "C" int lcn_debug_bn_bwd_fit(int F, int* blocks_out) {
+  LCN_REQUIRE(F == 64 || F == 128, "F=%d: the backward BatchNorm kernels run at F = 64 or 128", F);
+  const int P = LCN_J * F, ewy = ew_rows_per_block(P), threads = P / 8 * ewy;
+  int dev = 0, sm_regs = 0, sm_smem = 0, reserved = 0, sm_threads = 0, sm_blocks = 0;
+  LCN_CHECK_CUDA(cudaGetDevice(&dev));
+  LCN_CHECK_CUDA(cudaDeviceGetAttribute(&sm_regs, cudaDevAttrMaxRegistersPerMultiprocessor, dev));
+  LCN_CHECK_CUDA(cudaDeviceGetAttribute(&sm_smem, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev));
+  LCN_CHECK_CUDA(cudaDeviceGetAttribute(&reserved, cudaDevAttrReservedSharedMemoryPerBlock, dev));
+  LCN_CHECK_CUDA(cudaDeviceGetAttribute(&sm_threads, cudaDevAttrMaxThreadsPerMultiProcessor, dev));
+  LCN_CHECK_CUDA(cudaDeviceGetAttribute(&sm_blocks, cudaDevAttrMaxBlocksPerMultiprocessor, dev));
+  constexpr int kSubPartitions = 4, kRegUnit = 256;           // registers are allocated per warp in units of 256
+  auto warp_regs = [](const cudaFuncAttributes& a) { return (a.numRegs * 32 + kRegUnit - 1) / kRegUnit * kRegUnit; };
+  auto fit = [&](const cudaFuncAttributes& w, size_t w_dyn, int w_threads, const cudaFuncAttributes& k, size_t k_dyn) {
+    const int w_warps = (w_threads + 31) / 32, k_warps = (threads + 31) / 32;
+    const int sp_left = sm_regs / kSubPartitions - (w_warps + kSubPartitions - 1) / kSubPartitions * warp_regs(w);
+    const int by_regs = sp_left / warp_regs(k) * kSubPartitions / k_warps;
+    const long smem_left = (long)sm_smem - (long)(w.sharedSizeBytes + w_dyn + reserved);
+    const int by_smem = (int)(smem_left / (long)(k.sharedSizeBytes + k_dyn + reserved));
+    const int by_threads = (sm_threads - w_warps * 32) / (k_warps * 32);
+    return std::max(0, std::min(std::min(by_regs, by_smem), std::min(by_threads, sm_blocks - 1)));
+  };
+  const size_t reduce_dyn = bn_bwd_reduce_smem(P, ewy), apply_dyn = bn_bwd_apply_smem(P, ewy);
+  for (int x3 = 0; x3 < 2; ++x3) {
+    cudaFuncAttributes w, k[3];
+    size_t w_dyn = 0;
+    int w_threads = 0;
+    int rc = lcn_tc_wgrad_footprint(x3 != 0, &w, &w_dyn, &w_threads);
+    if (rc) return rc;
+    if (x3) {
+      LCN_CHECK_CUDA(cudaFuncGetAttributes(&k[0], k_bn_bwd_reduce<lcn_sp16>));
+      LCN_CHECK_CUDA(cudaFuncGetAttributes(&k[1], k_bn_bwd_apply<lcn_sp16, false>));
+      LCN_CHECK_CUDA(cudaFuncGetAttributes(&k[2], k_bn_bwd_apply<lcn_sp16, true>));
+    } else {
+      LCN_CHECK_CUDA(cudaFuncGetAttributes(&k[0], k_bn_bwd_reduce<__nv_bfloat16>));
+      LCN_CHECK_CUDA(cudaFuncGetAttributes(&k[1], k_bn_bwd_apply<__nv_bfloat16, false>));
+      LCN_CHECK_CUDA(cudaFuncGetAttributes(&k[2], k_bn_bwd_apply<__nv_bfloat16, true>));
+    }
+    for (int i = 0; i < 3; ++i) blocks_out[3 * x3 + i] = fit(w, w_dyn, w_threads, k[i], i == 0 ? reduce_dyn : apply_dyn);
+  }
+  return LCN_OK;
 }
 
 template <typename T>
